@@ -2,6 +2,7 @@
 """bench.py -- clip-frames/s of the TSCD aggregation stage (BASELINE.json metric) on N B200s.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|reference-gpu] [--config NAME] [--mode clips|long-clip]
+                  [--dump-outputs DIR]
   N > 1:  python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Configurations (--config; BASELINE.json `configs`):
@@ -165,6 +166,49 @@ def make_runner(cfg, dev):
         head, feats = views
         return st.forward(head, feats, torch.float16, te, B, F, L)
     return st, run
+
+
+# ------------------------------------------------------------------------------------------------- --dump-outputs
+DUMP_MAX_BYTES = 64_000_000
+NPY_HEADER_BYTES = 128             # np.save header of a 1-D / 2-D float array
+
+
+def caller_arrays(cfg, out, B):
+    """What a caller receives from one forward of the stage: {name: (per-frame list of float32 arrays or None, columns,
+    most rows a frame can hold)}.  TSCD stage: AggregationStage.to_lists (result / result_ori, per local frame [n,7] or None);
+    gen-1 stage: the refined class logits of each frame's proposals."""
+    from tscd_b200 import stage
+    if cfg.get("gen1"):
+        if int(out["status"].item()) != 0:
+            raise RuntimeError("the gen-1 stage reported a capacity error")
+        off = out["sel"]["row_off"][:B * cfg["F"] + 1].cpu().tolist()
+        logits = out["logits"][:off[-1]].cpu().numpy()
+        return {"logits": ([logits[a:b] for a, b in zip(off[:-1], off[1:])], logits.shape[1], out["sel"]["sel_rows"].shape[1])}
+    host = {k: out[k].cpu() for k in ("status", "det_count", "ori_count", "det_cand", "det_rows", "ori_rows")}
+    res, res_ori = stage.AggregationStage.to_lists(host, B, cfg["L"])
+    return {name: ([None if t is None else t.numpy() for t in lst], host[name + "_rows"].shape[2], host[name + "_rows"].shape[1])
+            for name, lst in (("det", res), ("ori", res_ori))}
+
+
+def dump_outputs(path, arrays, max_bytes=DUMP_MAX_BYTES, seed=0):
+    """Writes caller_arrays() to `path`: per name <name>_rows.npy (float32, the frames' rows concatenated in frame order) and
+    <name>_counts.npy (float64, rows per frame, -1 where the caller gets None); frames.npy (float64) lists the frames written.
+    When the frames could hold more than max_bytes at full capacity (headers included), a seeded sample of frames is written:
+    the first k of a permutation drawn from the frame count and the seed, k set by the output buffers' row capacity.  Two builds
+    with the same capacities dump the same frames; with different capacities one frame set contains the other."""
+    import numpy as np
+    n = len(next(iter(arrays.values()))[0])
+    frame_bytes = sum(cols * cap * 4 + 8 for _, cols, cap in arrays.values()) + 8
+    k = min(n, max(1, (max_bytes - NPY_HEADER_BYTES * (1 + 2 * len(arrays))) // frame_bytes))
+    frames = np.arange(n) if k == n else np.sort(np.random.default_rng(seed).permutation(n)[:k])
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "frames.npy"), frames.astype(np.float64))
+    for name, (lst, cols, _) in arrays.items():
+        picked = [lst[f] for f in frames]
+        rows = [a for a in picked if a is not None]
+        np.save(os.path.join(path, name + "_rows.npy"),
+                np.concatenate(rows).astype(np.float32) if rows else np.zeros((0, cols), np.float32))
+        np.save(os.path.join(path, name + "_counts.npy"), np.array([-1 if a is None else len(a) for a in picked], np.float64))
 
 
 # ------------------------------------------------------------------------------------------------- clocks
@@ -469,24 +513,27 @@ def run_ours(args, cfg, rank, world, local):
     torch.cuda.synchronize()
 
     # ---- one CUDA graph per input set (the stage has no host sync) ----
-    graphs = []
+    graphs, graph_outs = [], []
     if not args.no_graph:
         try:
             for i in range(nsets):
-                g, _ = st.capture_fn(lambda i=i: run(views[i], B, te)) if hasattr(st, "capture_fn") else _capture(lambda i=i: run(views[i], B, te), dev)
+                g, g_out = st.capture_fn(lambda i=i: run(views[i], B, te)) if hasattr(st, "capture_fn") else _capture(lambda i=i: run(views[i], B, te), dev)
                 graphs.append(g)
+                graph_outs.append(g_out)
             torch.cuda.synchronize()
         except Exception as e:   # noqa: BLE001
             sys.stderr.write(f"CUDA graph capture failed ({e}); timing eager launches\n")
-            graphs = []
+            graphs, graph_outs = [], []
             torch.cuda.synchronize()
 
     def step():
         for r in range(R):
             if graphs:
                 graphs[r % nsets].replay()
+                res = graph_outs[r % nsets]
             else:
-                run(views[r % nsets], B, te)
+                res = run(views[r % nsets], B, te)
+        return res
 
     for _ in range(args.warmup):
         step()
@@ -495,13 +542,16 @@ def run_ours(args, cfg, rank, world, local):
     clocks.start()
     barrier()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    last = None
     e0.record()
     for _ in range(args.steps):
-        step()
+        last = step()
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
     clk = clocks.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, caller_arrays(cfg, last, B))
     if world > 1:
         t = torch.tensor([ms], device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -526,7 +576,7 @@ def run_ours(args, cfg, rank, world, local):
     # ---- e2e: host (pinned) inputs -> detections on the host ----
     e2e = None
     if not cfg.get("gen1") and not args.no_e2e:
-        del graphs, sets, views, out
+        del graphs, graph_outs, last, sets, views, out
         torch.cuda.empty_cache()
         e2e = run_e2e(args, cfg, st, dev, rank, world, dist, barrier)
 
@@ -635,11 +685,11 @@ def run_e2e(args, cfg, st, dev, rank, world, dist, barrier):
     link = ClockSampler(torch.cuda.current_device(), extra="pstate,pcie.link.gen.current,pcie.link.width.current", period_ms=25)
     link.start()
     t0 = time.perf_counter()
-    e2e_steps = max(3, min(args.steps, 10)) * depth
+    e2e_calls = args.steps * depth                                   # --steps steps of `depth` calls each
     # throughput: `depth` calls in flight (double buffering): the PCIe phases of step i+1 overlap the compute tail and the host-side
     # unpacking of step i.  Every step's copies, kernels, read-back and unpacking happen inside the timed region.
     inflight = []
-    for i in range(e2e_steps):
+    for i in range(e2e_calls):
         inflight.append(submit(i))
         if len(inflight) == depth:
             res, res_ori, h2d, d2h = st.forward_host_collect(inflight.pop(0))
@@ -663,9 +713,9 @@ def run_e2e(args, cfg, st, dev, rank, world, dist, barrier):
         ev1.record()
         torch.cuda.synchronize()
         gpu_ms = ev0.elapsed_time(ev1)
-    return {"value": world * Be * F * e2e_steps / e2e_s, "unit": "clip-frames/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
-            "ms_per_call": 1e3 * e2e_s / e2e_steps, "gpu_ms_per_call": gpu_ms, "sync_call_ms": call_ms, "sync_call_split_ms": call_split, "plans_built": getattr(st, "host_plan_builds", None), "host": _host_info(), "warmup_calls": warm_calls, "gpu_state": link_state,
-            "clips_per_gpu_per_step": Be, "chunk_clips": args.e2e_chunk, "steps": e2e_steps, "calls_in_flight": depth,
+    return {"value": world * Be * F * e2e_calls / e2e_s, "unit": "clip-frames/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
+            "ms_per_call": 1e3 * e2e_s / e2e_calls, "gpu_ms_per_call": gpu_ms, "sync_call_ms": call_ms, "sync_call_split_ms": call_split, "plans_built": getattr(st, "host_plan_builds", None), "host": _host_info(), "warmup_calls": warm_calls, "gpu_state": link_state,
+            "clips_per_gpu_per_step": Be, "chunk_clips": args.e2e_chunk, "steps": args.steps, "calls": e2e_calls, "calls_in_flight": depth,
             "host_resident_input_bytes_per_step": nbytes(host),
             "note": "inputs are pinned HOST tensors; h2d counts the copied logits plus the rows read in place over PCIe"}
 
@@ -679,7 +729,7 @@ def run_sweep(args, rank, world, local):
         for K in SWEEP_K:
             cfg = dict(base, pre_k=P, top_k=K, workload=f"sweep point: pre-NMS top-{P} -> {K} proposals/frame, 64 clips x 32 frames per replay")
             a = argparse.Namespace(**vars(args))
-            a.replays, a.steps, a.warmup = args.replays or 4, min(args.steps, 5), 3
+            a.replays, a.warmup = args.replays or 4, 3
             line = run_ours(a, cfg, rank, world, local)
             if line is not None:
                 pt = {"P": P, "K": K, "value": line["value"], "ms_per_replay": line["ms_per_step"] / a.replays,
@@ -695,7 +745,8 @@ def run_sweep(args, rank, world, local):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps; the e2e leg times as many steps of --e2e-depth calls, "
+                    "the sweep as many steps per point")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference", "reference-gpu"])
     ap.add_argument("--config", default="ovis_a_k30", choices=list(CONFIGS) + ["sweep"])
@@ -712,7 +763,14 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="launch eagerly instead of replaying CUDA graphs")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline / reference-gpu legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last graph replay of the last step "
+                    "returned to its caller as DIR/<name>.npy (float32 / float64, at most 64,000,000 bytes; rank 0 only); inputs are seeded, "
+                    "so runs with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.mode != "clips" or args.config == "sweep" or args.impl != "ours"):
+        ap.error("--dump-outputs applies to the timed stage: --impl ours, --mode clips, a single --config")
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
     if args.mode == "long-clip":
