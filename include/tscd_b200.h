@@ -38,6 +38,11 @@ extern "C" {
 
 #define TSCD_MAX_LEVELS 3
 
+/* Per-frame proposal capacity of the aggregation kernels.  Up to 512 proposals per frame (the default tier) every kernel
+ * runs the paths it always has; the wide tier (513 .. TSCD_MAX_PROPOSALS) takes the CTA-cooperative LSAP solver of
+ * tscd_cafm_lap and the global-memory merge of tscd_nms (cand_cap > 16384).  Mirrored by tscd_b200.selection.MAX_PROPOSALS. */
+#define TSCD_MAX_PROPOSALS 2048
+
 /* Strided view of one per-anchor quantity with `channels` channels over up to 3 FPN levels.
  * element(frame f, level l, local anchor a, channel c) = ptr[l] + f*frame_stride[l] + a*anchor_stride[l]
  *                                                        + c*chan_stride[l]            (strides in elements)
@@ -142,7 +147,11 @@ int tscd_debug_select_keys(const unsigned short* half_bits, int n, int apply_sig
  *   partition, one CTA per (frame, class) greedy NMS (exact whenever no cross-class pair of offset boxes exceeds the
  *   threshold, which is tested explicitly), per-frame score-ordered merge; frames that fail the test take an exact general
  *   path.  `ws` must then hold tscd_nms_workspace_bytes(num_frames, cand_cap) bytes.
- * cand_cap > 16384 returns TSCD_ERR_CAPACITY from the call itself. */
+ *   16384 < cand_cap <= 65536 (wide tier: 2048 proposals x 30 classes = 61 440 rows): the same partition and per-class kernels,
+ *   then the merge goes through the workspace -- runs of 16384 positions sorted in shared memory, each entry ranked against the
+ *   other runs by binary search; frames that fail the cross-class test run the general path over the merged order in global
+ *   memory.  Same keep lists, same workspace contract (tscd_nms_workspace_bytes grows by 20 bytes per candidate row).
+ * cand_cap > 65536 returns TSCD_ERR_CAPACITY from the call itself. */
 typedef struct {
     int32_t num_frames;
     int32_t cand_cap;     /* row pitch of the candidate arrays */
@@ -406,7 +415,9 @@ typedef struct {
     const float* st_reg; const float* st_cls; const float* st_nreg; const float* st_ncls;
     float* cost;                 /* [B*L, kmax, kmax] */
     int32_t* ref_n;              /* [B*L] rows on the reference side of every frame's matching (0 for empty frames) */
-    /* TSCD_F32 (0): emb_* / norm_* as declared above (fp32 FMA kernel, any kmax <= 512).  TSCD_F16 / TSCD_BF16 (kmax <= 32): emb_reg /
+    /* kmax <= TSCD_MAX_PROPOSALS; above 512 only the 16-bit-copy kernel below (emb_dtype TSCD_F32 with emb_reg16 / emb_cls16 set),
+     * anything else returns TSCD_ERR_UNSUPPORTED.
+     * TSCD_F32 (0): emb_* / norm_* as declared above (fp32 FMA kernel, any kmax <= 512).  TSCD_F16 / TSCD_BF16 (kmax <= 32): emb_reg /
      * emb_cls point to 16-bit [loc_cap, 4D] embeddings (the GEMM outputs as the tensor cores produced them), the costs run on
      * mma.sync with fp32 accumulation and norm_reg / norm_cls are OUTPUTS (written for the rows of every frame) */
     int32_t emb_dtype;
@@ -423,7 +434,10 @@ int tscd_cafm_cost(const tscd_cafm_cost_args* args, void* stream);
 /* Rectangular LSAP of every frame's cost table in parallel (one warp per frame; scipy.optimize.
  * linear_sum_assignment semantics, fp64).  The assignment of a frame does not depend on the order in which the
  * previous frame remembers its rows, so all frames are solved before the sequential chain, which only re-indexes:
- * lap_col[lf][r] = matched column of reference row r (-1: none), lap_row[lf][c] = matched reference row of column c. */
+ * lap_col[lf][r] = matched column of reference row r (-1: none), lap_row[lf][c] = matched reference row of column c.
+ * kmax <= TSCD_MAX_PROPOSALS.  Problems with max(ref_n, n) <= 512 are solved by one warp each exactly as before; larger ones (wide
+ * tier) by one 512-thread CTA each (CTA-cooperative column scan and arg-min, fp64 potentials, state in ~42 x kmax bytes of shared
+ * memory), with the same scan order and tie rules, i.e. SciPy's assignment.  The solver is chosen per problem on the device. */
 typedef struct {
     int32_t num_frames, kmax;
     const int32_t* lrow_off;
@@ -496,6 +510,8 @@ int tscd_cafm_chain(const tscd_cafm_chain_args* args, void* stream);
  * ranges q_beg/q_end/kv_beg/kv_end, keys / values = the k_reg / v_reg projections) into `attn`, then phase 2 (identity +
  * LayerNorms, outputs, state);  phase 3 once (matching embeddings into the carried state).  `base` is the argument block of
  * tscd_cafm_chain: feat / edge / kin (fp32), lap_*, state and output fields are used; kproj*, vproj*, wq*, sc_* are not. */
+/* tscd_cafm_wide accepts kmax <= TSCD_MAX_PROPOSALS (tscd_cafm_chain itself stays at kmax <= 512); the permutation kernel walks
+ * the frame's rows in chunks of 512, so frames of up to 2048 proposals keep the same row order and state layout. */
 typedef struct {
     tscd_cafm_chain_args base;
     void* qin16;             /* out (phase 1) [B*kmax, D] 16-bit (out_dtype) */

@@ -20,7 +20,8 @@
 namespace tscd {
 
 constexpr int kChainThreads = 512;
-constexpr int kChainMax = 512;
+constexpr int kChainMax = 512;                   // default tier: the one-warp LSAP, the generic one-CTA chain
+constexpr int kWideMax = TSCD_MAX_PROPOSALS;     // wide tier: CTA LSAP, wide chain, wide cost kernel
 constexpr int kCostSmem = 64 * 64;
 
 __device__ __forceinline__ float se_gate(float a, float b, const float* w1, const float* w2) {
@@ -687,7 +688,7 @@ __global__ void __launch_bounds__(32) cafm_lap_kernel(const tscd_cafm_lap_args a
     const int lf = blockIdx.x, lane = threadIdx.x;
     const int n = a.lrow_off[lf + 1] - a.lrow_off[lf];
     const int np = a.ref_n[lf];
-    if (n <= 0 || np <= 0) return;
+    if (n <= 0 || np <= 0 || max(n, np) > kChainMax) return;      // wide problems: cafm_lap_cta_kernel
     const int KM = a.kmax;
     const float* C = a.cost + (int64_t)lf * KM * KM;
     int ldc = KM;
@@ -721,6 +722,130 @@ __global__ void __launch_bounds__(32) cafm_lap_kernel(const tscd_cafm_lap_args a
     } else {                      // transposed problem: its rows are the current columns
         for (int r = lane; r < np; r += 32) col[r] = s.row4col[r];
         for (int c = lane; c < n; c += 32) row[c] = s.col4row[c];
+    }
+}
+
+// Wide problems (max(n_prev, n) > kChainMax, up to kWideMax): the same shortest-augmenting-path algorithm with the whole
+// CTA on every Dijkstra step.  The column scan is spread over the block; the arg-min is a warp reduction of (value, tie key)
+// followed by warp 0 over the per-warp winners, which also removes the winner from `remaining` (swap with the last entry)
+// before the second barrier of the step.  Tie keys are those of lap_warp (an unassigned column wins, the LAST one in scan
+// order; otherwise the FIRST minimum), so the result is SciPy's assignment, not only its cost.  State in shared memory,
+// sized by kmax: fp64 potentials u / v and path costs, path / col4row / row4col / remaining, SR / SC flags (86 KB at 2048).
+constexpr int kLapCtaThreads = 512;
+
+__global__ void __launch_bounds__(kLapCtaThreads, 1) cafm_lap_cta_kernel(const tscd_cafm_lap_args a) {
+    extern __shared__ __align__(16) unsigned char lap_smem[];
+    constexpr int NW = kLapCtaThreads / 32;
+    __shared__ double red_v[NW];
+    __shared__ unsigned red_tb[NW];
+    __shared__ double bc_min;
+    __shared__ int bc_j, bc_r4c;
+    const int lf = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int n = a.lrow_off[lf + 1] - a.lrow_off[lf];
+    const int np = a.ref_n[lf];
+    if (n <= 0 || np <= 0 || max(n, np) <= kChainMax) return;     // default-tier problems: cafm_lap_kernel
+    const int KM = a.kmax;
+    double* u = reinterpret_cast<double*>(lap_smem);
+    double* v = u + KM;
+    double* spc = v + KM;
+    int* path = reinterpret_cast<int*>(spc + KM);
+    int* col4row = path + KM;
+    int* row4col = col4row + KM;
+    int* remaining = row4col + KM;
+    unsigned char* SR = reinterpret_cast<unsigned char*>(remaining + KM);
+    unsigned char* SC = SR + KM;
+    const float* C = a.cost + (int64_t)lf * KM * KM;
+    const bool tr = n < np;
+    const int nr = tr ? n : np, nc = tr ? np : n;
+    for (int j = tid; j < nc; j += kLapCtaThreads) { v[j] = 0.0; row4col[j] = -1; path[j] = -1; }
+    for (int i = tid; i < nr; i += kLapCtaThreads) { u[i] = 0.0; col4row[i] = -1; }
+    __syncthreads();
+    for (int cur = 0; cur < nr; ++cur) {
+        for (int it = tid; it < nc; it += kLapCtaThreads) { remaining[it] = nc - it - 1; spc[it] = INFINITY; SC[it] = 0; }
+        for (int i = tid; i < nr; i += kLapCtaThreads) SR[i] = (i == cur) ? 1 : 0;
+        __syncthreads();
+        double min_val = 0.0;
+        int i = cur, num_rem = nc, sink = -1;
+        while (sink == -1) {
+            const double ui = u[i];
+            double best = INFINITY;
+            unsigned best_tb = 0xffffffffu;
+            for (int it = tid; it < num_rem; it += kLapCtaThreads) {
+                const int j = remaining[it];
+                const double c = (double)(tr ? C[(int64_t)j * KM + i] : C[(int64_t)i * KM + j]);
+                const double r = min_val + c - ui - v[j];
+                if (r < spc[j]) { path[j] = i; spc[j] = r; }
+                const double sj = spc[j];
+                const unsigned tb = (row4col[j] == -1) ? (unsigned)(0xffff - it) : (0x10000u | (unsigned)it);
+                if (sj < best || (sj == best && tb < best_tb)) { best = sj; best_tb = tb; }
+            }
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) {
+                const double ob = __shfl_xor_sync(0xffffffffu, best, o);
+                const unsigned otb = __shfl_xor_sync(0xffffffffu, best_tb, o);
+                if (ob < best || (ob == best && otb < best_tb)) { best = ob; best_tb = otb; }
+            }
+            if (lane == 0) { red_v[warp] = best; red_tb[warp] = best_tb; }
+            __syncthreads();
+            if (warp == 0) {
+                best = lane < NW ? red_v[lane] : INFINITY;
+                best_tb = lane < NW ? red_tb[lane] : 0xffffffffu;
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) {
+                    const double ob = __shfl_xor_sync(0xffffffffu, best, o);
+                    const unsigned otb = __shfl_xor_sync(0xffffffffu, best_tb, o);
+                    if (ob < best || (ob == best && otb < best_tb)) { best = ob; best_tb = otb; }
+                }
+                if (lane == 0) {
+                    const int best_it = (best_tb == 0xffffffffu) ? -1 : ((best_tb & 0x10000u) ? (int)(best_tb & 0xffffu) : 0xffff - (int)best_tb);
+                    bc_min = best;
+                    if (best_it < 0 || best == INFINITY) {
+                        bc_j = -1;
+                    } else {
+                        const int j = remaining[best_it];
+                        bc_j = j;
+                        bc_r4c = row4col[j];
+                        SC[j] = 1;
+                        remaining[best_it] = remaining[num_rem - 1];
+                        if (row4col[j] != -1) SR[row4col[j]] = 1;
+                    }
+                }
+            }
+            __syncthreads();
+            min_val = bc_min;
+            const int j = bc_j;
+            if (j < 0 || min_val == INFINITY) { sink = -2; break; }     // infeasible (cannot happen: finite costs)
+            if (bc_r4c == -1) sink = j; else i = bc_r4c;
+            --num_rem;
+        }
+        if (sink < 0) break;
+        for (int r = tid; r < nr; r += kLapCtaThreads)
+            if (r == cur) u[r] += min_val;
+            else if (SR[r]) u[r] += min_val - spc[col4row[r]];
+        for (int j = tid; j < nc; j += kLapCtaThreads)
+            if (SC[j]) v[j] -= min_val - spc[j];
+        __syncthreads();
+        if (tid == 0) {
+            int j = sink;
+            for (;;) {
+                const int r = path[j];
+                row4col[j] = r;
+                const int t = col4row[r];
+                col4row[r] = j;
+                j = t;
+                if (r == cur) break;
+            }
+        }
+        __syncthreads();
+    }
+    int32_t* col = a.lap_col + (int64_t)lf * KM;
+    int32_t* row = a.lap_row + (int64_t)lf * KM;
+    if (!tr) {
+        for (int r = tid; r < np; r += kLapCtaThreads) col[r] = col4row[r];
+        for (int c = tid; c < n; c += kLapCtaThreads) row[c] = row4col[c];
+    } else {                      // transposed problem: its rows are the current columns
+        for (int r = tid; r < np; r += kLapCtaThreads) col[r] = row4col[r];
+        for (int c = tid; c < n; c += kLapCtaThreads) row[c] = col4row[c];
     }
 }
 
@@ -1404,7 +1529,7 @@ __global__ void cafm_wide_begin_kernel(const tscd_cafm_wide_args w) {
     if (threadIdx.x == 0) { w.n_prev[b] = resume ? a.st_n[b] : 0; w.last_l0[b] = -1; }
 }
 
-// one CTA (512 threads >= kmax) per clip: control block + perm / prow of frame f (tscd_matching.py:813-844)
+// one CTA (512 threads, rows in chunks of 512) per clip: control block + perm / prow of frame f (tscd_matching.py:813-844)
 __global__ void __launch_bounds__(512) cafm_wide_perm_kernel(const tscd_cafm_wide_args w, int f) {
     __shared__ int scan[40];
     const tscd_cafm_chain_args& a = w.base;
@@ -1418,7 +1543,7 @@ __global__ void __launch_bounds__(512) cafm_wide_perm_kernel(const tscd_cafm_wid
     int* prow = w.prow_s + (int64_t)b * KM;
     const int* ord = w.ord_prev + (int64_t)b * KM;
     __syncthreads();                                 // every thread has read n_prev before thread 0 may reset it
-    if (n == 0 || n > KM || n > kChainMax || n_prev > KM) {
+    if (n == 0 || n > KM || n > kWideMax || n_prev > KM) {
         if (tid == 0) {
             if (n == 0) { if (f == 0 && !resume) w.n_prev[b] = 0; }
             else atomicMin(a.status, TSCD_ERR_CAPACITY);
@@ -1431,20 +1556,29 @@ __global__ void __launch_bounds__(512) cafm_wide_perm_kernel(const tscd_cafm_wid
     const int np = first ? n : n_prev;
     const int32_t* colo = a.lap_col + (int64_t)lf * KM;
     const int32_t* rowo = a.lap_row + (int64_t)lf * KM;
+    int carry = 0;
     if (np <= n) {
-        if (tid < np) { perm[tid] = colo[first ? tid : ord[tid]]; prow[tid] = tid; }
+        for (int r = tid; r < np; r += 512) { perm[r] = colo[first ? r : ord[r]]; prow[r] = r; }
         // unmatched current columns follow in ascending order
-        const int flag = (tid < n && rowo[tid] == -1) ? 1 : 0;
-        int tot;
-        const int ex = block_excl_scan(flag, scan, &tot);
-        if (flag && np + ex < n) { perm[np + ex] = tid; prow[np + ex] = -1 - tid; }
+        for (int c0 = 0; c0 < n; c0 += 512) {
+            const int c = c0 + tid;
+            const int flag = (c < n && rowo[c] == -1) ? 1 : 0;
+            int tot;
+            const int ex = carry + block_excl_scan(flag, scan, &tot);
+            if (flag && np + ex < n) { perm[np + ex] = c; prow[np + ex] = -1 - c; }
+            carry += tot;
+        }
     } else {
-        int c = -1;
-        if (tid < np) c = colo[ord[tid]];
-        const int flag = c >= 0 ? 1 : 0;
-        int tot;
-        const int ex = block_excl_scan(flag, scan, &tot);
-        if (flag && ex < n) { perm[ex] = c; prow[ex] = tid; }
+        for (int r0 = 0; r0 < np; r0 += 512) {
+            const int r = r0 + tid;
+            int c = -1;
+            if (r < np) c = colo[ord[r]];
+            const int flag = c >= 0 ? 1 : 0;
+            int tot;
+            const int ex = carry + block_excl_scan(flag, scan, &tot);
+            if (flag && ex < n) { perm[ex] = c; prow[ex] = r; }
+            carry += tot;
+        }
     }
     if (tid == 0) {
         ctl->n = n; ctl->np = np; ctl->first = first ? 1 : 0; ctl->l0 = l0; ctl->skip = 0;
@@ -1556,7 +1690,7 @@ extern "C" int tscd_cafm_wide(const tscd_cafm_wide_args* w, int phase, int frame
     using namespace tscd;
     if (!w) return TSCD_ERR_INVALID_ARG;
     const tscd_cafm_chain_args& a = w->base;
-    if (a.B <= 0 || a.L <= 0 || a.D != 256 || a.kmax <= 0 || a.kmax > kChainMax || frame < 0 || frame >= a.L) return TSCD_ERR_INVALID_ARG;
+    if (a.B <= 0 || a.L <= 0 || a.D != 256 || a.kmax <= 0 || a.kmax > kWideMax || frame < 0 || frame >= a.L) return TSCD_ERR_INVALID_ARG;
     if (a.emb_dtype != TSCD_F32 || !w->ctl || !w->perm_s || !w->prow_s || !w->ord_prev || !w->n_prev || !w->last_l0 || !w->q_beg ||
         !w->q_end || !w->kv_beg || !w->kv_end || !w->qin16 || !w->attn)
         return TSCD_ERR_INVALID_ARG;
@@ -1600,7 +1734,9 @@ extern "C" int tscd_cafm_prep(const tscd_cafm_prep_args* a, void* stream) {
 
 extern "C" int tscd_cafm_cost(const tscd_cafm_cost_args* a, void* stream) {
     using namespace tscd;
-    if (!a || a->B <= 0 || a->L <= 0 || a->D != 256 || a->kmax <= 0 || a->kmax > kChainMax) return TSCD_ERR_INVALID_ARG;
+    if (!a || a->B <= 0 || a->L <= 0 || a->D != 256 || a->kmax <= 0 || a->kmax > kWideMax) return TSCD_ERR_INVALID_ARG;
+    // above kChainMax only the tensor-core kernel of the wide frames (16-bit copies of the embeddings)
+    if (a->kmax > kChainMax && (a->emb_dtype != TSCD_F32 || !a->emb_reg16 || !a->emb_cls16)) return TSCD_ERR_UNSUPPORTED;
     const int tiles = (a->kmax + 31) / 32;
     if (a->emb_dtype != TSCD_F32) {                        // 16-bit matching embeddings: tensor-core kernel, frames <= 32 proposals
         if (a->kmax > 32 || !a->norm_reg || !a->norm_cls || !a->ref_n) return TSCD_ERR_INVALID_ARG;
@@ -1633,7 +1769,7 @@ extern "C" int tscd_cafm_cost(const tscd_cafm_cost_args* a, void* stream) {
 
 extern "C" int tscd_cafm_lap(const tscd_cafm_lap_args* a, void* stream) {
     using namespace tscd;
-    if (!a || a->num_frames <= 0 || a->kmax <= 0 || a->kmax > kChainMax) return TSCD_ERR_INVALID_ARG;
+    if (!a || a->num_frames <= 0 || a->kmax <= 0 || a->kmax > kWideMax) return TSCD_ERR_INVALID_ARG;
     if (a->kmax <= 32) {
         const size_t sm = (size_t)kLapPack * 1024 * sizeof(float);
         if (cudaFuncSetAttribute(cafm_lap_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm) != cudaSuccess) return TSCD_ERR_CUDA;
@@ -1645,6 +1781,12 @@ extern "C" int tscd_cafm_lap(const tscd_cafm_lap_args* a, void* stream) {
     if (cudaFuncSetAttribute(cafm_lap_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return TSCD_ERR_CUDA;
     cafm_lap_kernel<<<a->num_frames, 32, smem, reinterpret_cast<cudaStream_t>(stream)>>>(*a);
     TSCD_CUDA_CHECK_LAUNCH();
+    if (a->kmax > kChainMax) {       // the solver is picked per problem on the device: each kernel skips the other's problems
+        const size_t smem_w = (size_t)a->kmax * (3 * sizeof(double) + 4 * sizeof(int) + 2);
+        if (cudaFuncSetAttribute(cafm_lap_cta_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_w) != cudaSuccess) return TSCD_ERR_CUDA;
+        cafm_lap_cta_kernel<<<a->num_frames, kLapCtaThreads, smem_w, reinterpret_cast<cudaStream_t>(stream)>>>(*a);
+        TSCD_CUDA_CHECK_LAUNCH();
+    }
     return TSCD_OK;
 }
 

@@ -1,12 +1,13 @@
 // Shared pieces of the NMS kernels (csrc/nms.cu: frames of up to 4096 candidates in shared memory; csrc/nms_large.cu:
-// up to 16384 candidates through a global-memory workspace).
+// up to 65536 candidates through a global-memory workspace).
 #pragma once
 #include "common.cuh"
 
 namespace tscd {
 
 constexpr int kNmsCap = 4096;          // one-CTA-per-frame kernels (shared-memory sort)
-constexpr int kNmsLargeCap = 16384;    // workspace path
+constexpr int kNmsLargeCap = 16384;    // workspace path, per-frame merge in one CTA's shared memory
+constexpr int kNmsWideCap = 65536;     // workspace path, merge through global memory (wide tier: 2048 proposals x <= 32 classes)
 
 // torchvision's nms predicate on two (offset) boxes: inter / (Sa + Sb - inter) > thr, every operation rounded to nearest
 // single precision exactly once (no FMA contraction), the comparison in double like the CPU kernel.

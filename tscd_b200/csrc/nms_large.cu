@@ -14,6 +14,16 @@
 //   nmsl_merge      one CTA per frame: sort the kept candidates by (score desc, position asc) -> keep list.  Marked frames
 //                   (cross-class hit, class ids outside [0,256), a class of more than kClassCap members) are redone with
 //                   the general algorithm: full sort + lazy greedy over all candidates (slow, exact).
+//
+// Frames of more than 16384 candidates (up to 65536: the wide tier's 2048 proposals x 30 classes = 61 440 rows) keep the
+// first two kernels; their candidates no longer fit one CTA's sort, so the merge goes through global memory:
+//   nmsw_run        one CTA per (frame, run of 16384 positions): the run's kept candidates (every candidate of a marked frame)
+//                   sorted by (score desc, position asc) in shared memory, written to the workspace;
+//   nmsw_rank       one thread per sorted entry: its rank in the frame = its rank in its run + the number of larger keys in
+//                   each other run (binary search; keys are unique, they carry the position) -> the merged order, and the keep
+//                   list of an unmarked frame;
+//   nmsw_final      one CTA per frame: keep count / overflow status, and for marked frames the general algorithm's lazy
+//                   greedy over the merged order in global memory.
 #include "nms.cuh"
 
 namespace tscd {
@@ -21,6 +31,8 @@ namespace tscd {
 constexpr int kClassCap = 2048;        // members of one class handled by nmsl_class
 constexpr int kPartThreads = 512, kClassThreads = 256, kMergeThreads = 1024;
 constexpr int kClassSlots = 32;        // grid.y of nmsl_class: classes are dealt round-robin over the slots
+
+constexpr int kRun = 16384, kRunsMax = kNmsWideCap / kRun;   // wide path: sorted runs per frame
 
 struct LargeWs {
     float* off_unit;        // [F]
@@ -32,13 +44,20 @@ struct LargeWs {
     unsigned char* ids;     // [F][256]
     int* list;              // [F][cap]
     unsigned char* flag;    // [F][cap]
+    // wide path only (cap > kNmsLargeCap)
+    int* run_n;                     // [F][kRunsMax] entries of every run
+    unsigned long long* run_key;    // [F][cap] run r at [r * kRun, r * kRun + run_n)
+    unsigned long long* merged;     // [F][cap] every run's entries in frame order
+    int* kept;                      // [F][cap] marked frames: merged ranks of the boxes kept so far
 };
 
 __host__ __device__ inline size_t r16(size_t x) { return (x + 15) & ~(size_t)15; }
 
 __host__ inline size_t large_ws_bytes(int F, int cap) {
-    return r16((size_t)F * 4) * 3 + r16((size_t)F * 257 * 4) + r16((size_t)F * 256 * 4) * 2 + r16((size_t)F * 256) +
-           r16((size_t)F * cap * 4) + r16((size_t)F * cap);
+    size_t b = r16((size_t)F * 4) * 3 + r16((size_t)F * 257 * 4) + r16((size_t)F * 256 * 4) * 2 + r16((size_t)F * 256) +
+               r16((size_t)F * cap * 4) + r16((size_t)F * cap);
+    if (cap > kNmsLargeCap) b += r16((size_t)F * kRunsMax * 4) + 2 * r16((size_t)F * cap * 8) + r16((size_t)F * cap * 4);
+    return b;
 }
 __host__ inline LargeWs carve_large_ws(void* p, int F, int cap) {
     unsigned char* c = reinterpret_cast<unsigned char*>(p);
@@ -51,7 +70,14 @@ __host__ inline LargeWs carve_large_ws(void* p, int F, int cap) {
     w.hi = reinterpret_cast<float*>(c); c += r16((size_t)F * 256 * 4);
     w.ids = c; c += r16((size_t)F * 256);
     w.list = reinterpret_cast<int*>(c); c += r16((size_t)F * cap * 4);
-    w.flag = c;
+    w.flag = c; c += r16((size_t)F * cap);
+    w.run_n = nullptr; w.run_key = nullptr; w.merged = nullptr; w.kept = nullptr;
+    if (cap > kNmsLargeCap) {
+        w.run_n = reinterpret_cast<int*>(c); c += r16((size_t)F * kRunsMax * 4);
+        w.run_key = reinterpret_cast<unsigned long long*>(c); c += r16((size_t)F * cap * 8);
+        w.merged = reinterpret_cast<unsigned long long*>(c); c += r16((size_t)F * cap * 8);
+        w.kept = reinterpret_cast<int*>(c);
+    }
     return w;
 }
 
@@ -364,8 +390,156 @@ __global__ void __launch_bounds__(kMergeThreads) nmsl_merge_kernel(const tscd_nm
     }
 }
 
+// ------------------------------------------------------------------------------------------------ wide merge (> 16384)
+__global__ void __launch_bounds__(kMergeThreads) nmsw_run_kernel(const tscd_nms_args args, const LargeWs ws) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    unsigned long long* skey = reinterpret_cast<unsigned long long*>(smem_raw);      // [kRun]
+    __shared__ int s_cnt;
+    const int frame = blockIdx.x, run = blockIdx.y, tid = threadIdx.x;
+    const int n = min(args.count[frame], args.cand_cap);
+    const int lo = run * kRun, hi = min(lo + kRun, n);
+    const int64_t base = (int64_t)frame * args.cand_cap;
+    if (hi <= lo) {
+        if (tid == 0) ws.run_n[frame * kRunsMax + run] = 0;
+        return;
+    }
+    const bool all = ws.fallback[frame] != 0;          // marked frame: the general path orders every candidate
+    const float* gscore = args.score + base;
+    const unsigned char* flag = ws.flag + base;
+    if (tid == 0) s_cnt = 0;
+    __syncthreads();
+    for (int i = lo + tid; i < hi; i += blockDim.x)
+        if (all || flag[i]) skey[atomicAdd(&s_cnt, 1)] = nms_key(gscore[i], i);
+    __syncthreads();
+    const int k = s_cnt;
+    int cap = kMergeThreads;
+    while (cap < k) cap <<= 1;
+    block_sort_desc64_dyn<unsigned long long>(skey, k, cap);
+    unsigned long long* out = ws.run_key + base + lo;
+    for (int j = tid; j < k; j += blockDim.x) out[j] = skey[j];
+    if (tid == 0) ws.run_n[frame * kRunsMax + run] = k;
+}
+
+__global__ void __launch_bounds__(256) nmsw_rank_kernel(const tscd_nms_args args, const LargeWs ws) {
+    const int frame = blockIdx.y;
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;          // entry e of run e / kRun
+    const int run = e / kRun, t = e - run * kRun;
+    if (run >= kRunsMax || (int64_t)run * kRun >= args.cand_cap) return;
+    const int* rn = ws.run_n + frame * kRunsMax;
+    if (t >= rn[run]) return;
+    const int64_t base = (int64_t)frame * args.cand_cap;
+    const unsigned long long key = ws.run_key[base + e];
+    int rank = t;
+    for (int r = 0; r < kRunsMax && (int64_t)r * kRun < args.cand_cap; ++r) {
+        if (r == run) continue;
+        const unsigned long long* rk = ws.run_key + base + (int64_t)r * kRun;
+        int lo = 0, hi = rn[r];                                    // descending run: count the entries > key
+        while (lo < hi) {
+            const int mid = (lo + hi) >> 1;
+            if (rk[mid] > key) lo = mid + 1; else hi = mid;
+        }
+        rank += lo;
+    }
+    ws.merged[base + rank] = key;
+    if (!ws.fallback[frame] && rank < args.max_keep) args.keep[(int64_t)frame * args.max_keep + rank] = key_pos(key);
+}
+
+// keep count of every frame; marked frames: nmsl_merge's general path with the sorted keys and the kept list in global memory
+__global__ void __launch_bounds__(kMergeThreads) nmsw_final_kernel(const tscd_nms_args args, const LargeWs ws) {
+    __shared__ int s_cnt;
+    __shared__ float4 cbox[32];
+    __shared__ float carea[32];
+    __shared__ unsigned int cmask[32];
+    __shared__ unsigned int s_deadbits;
+    const int frame = blockIdx.x, tid = threadIdx.x;
+    const int n = min(args.count[frame], args.cand_cap);
+    const int max_keep = args.max_keep;
+    int32_t* keep = args.keep + (int64_t)frame * max_keep;
+    if (n <= 0) {
+        if (tid == 0) args.keep_count[frame] = 0;
+        return;
+    }
+    const int64_t base = (int64_t)frame * args.cand_cap;
+    if (!ws.fallback[frame]) {
+        if (tid == 0) {
+            int k = 0;
+            for (int r = 0; r < kRunsMax && (int64_t)r * kRun < args.cand_cap; ++r) k += ws.run_n[frame * kRunsMax + r];
+            args.keep_count[frame] = min(k, max_keep);
+            if (args.strict_keep && k > max_keep) atomicMin(args.status, TSCD_ERR_CAPACITY);
+        }
+        return;
+    }
+    const unsigned long long* skey = ws.merged + base;
+    int* g_kept = ws.kept + base;
+    const float4* gbox = reinterpret_cast<const float4*>(args.box) + base;
+    const int32_t* gcls = args.cls + base;
+    const float off_unit = ws.off_unit[frame];
+    const double thr = (double)args.iou_thresh;
+    if (tid == 0) s_cnt = 0;
+    __syncthreads();
+    const int limit = args.strict_keep ? n : max_keep;   // strict: count every survivor to detect the overflow
+    for (int c0 = 0; c0 < n; c0 += 32) {
+        const int cn = min(32, n - c0);
+        if (tid < 32) {
+            cmask[tid] = 0u;
+            if (tid < cn) {
+                const int pos = key_pos(skey[c0 + tid]);
+                const float4 b = offset_box(gbox[pos], gcls[pos], off_unit);
+                cbox[tid] = b;
+                carea[tid] = box_area(b);
+            }
+        }
+        if (tid == 0) s_deadbits = 0u;
+        __syncthreads();
+        const int nk0 = s_cnt;
+        {
+            const int l = tid & 31;
+            if (l < cn) {
+                const float4 bl = cbox[l];
+                const float sl = carea[l];
+                bool dead = false;
+                for (int k = tid >> 5; k < nk0 && !dead; k += kMergeThreads / 32) {
+                    const int pos = key_pos(skey[g_kept[k]]);
+                    const float4 bk = offset_box(gbox[pos], gcls[pos], off_unit);
+                    if (fminf(bk.z, bl.z) > fmaxf(bk.x, bl.x)) dead = iou_gt(bk, box_area(bk), bl, sl, thr);
+                }
+                if (dead) atomicOr(&s_deadbits, 1u << l);
+            }
+        }
+        {
+            const int l = tid >> 5, j = tid & 31;        // 1024 threads = the 32 x 32 pairs of the chunk
+            if (j < l && l < cn && iou_gt(cbox[j], carea[j], cbox[l], carea[l], thr)) atomicOr(&cmask[l], 1u << j);
+        }
+        __syncthreads();
+        if (tid < 32) {
+            const int lane = tid;
+            const bool alive = (lane < cn) && !((s_deadbits >> lane) & 1u);
+            const unsigned alive_bits = __ballot_sync(0xffffffffu, alive);
+            const unsigned my = cmask[lane];
+            unsigned kb = 0u;
+#pragma unroll
+            for (int l = 0; l < 32; ++l) {
+                const unsigned mm = __shfl_sync(0xffffffffu, my, l);
+                if (((alive_bits >> l) & 1u) && !(mm & kb)) kb |= 1u << l;
+            }
+            const int rank = nk0 + __popc(kb & ((1u << lane) - 1u));
+            if ((kb >> lane) & 1u) {
+                g_kept[rank] = c0 + lane;
+                if (rank < max_keep) keep[rank] = key_pos(skey[c0 + lane]);
+            }
+            if (lane == 0) s_cnt = nk0 + __popc(kb);
+        }
+        __syncthreads();                                 // also orders the g_kept writes before the next chunk's reads
+        if (s_cnt >= limit) break;
+    }
+    if (tid == 0) {
+        args.keep_count[frame] = min(s_cnt, max_keep);
+        if (args.strict_keep && s_cnt > max_keep) atomicMin(args.status, TSCD_ERR_CAPACITY);
+    }
+}
+
 int nms_large_launch(const tscd_nms_args& a, cudaStream_t st) {
-    if (a.cand_cap > kNmsLargeCap) return TSCD_ERR_CAPACITY;
+    if (a.cand_cap > kNmsWideCap) return TSCD_ERR_CAPACITY;
     if (!a.ws || a.ws_bytes < (int64_t)large_ws_bytes(a.num_frames, a.cand_cap)) return TSCD_ERR_INVALID_ARG;
     const LargeWs ws = carve_large_ws(a.ws, a.num_frames, a.cand_cap);
     nmsl_partition_kernel<<<a.num_frames, kPartThreads, 0, st>>>(a, ws);
@@ -376,6 +550,18 @@ int nms_large_launch(const tscd_nms_args& a, cudaStream_t st) {
     if (cudaFuncSetAttribute(nmsl_class_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_c) != cudaSuccess) return TSCD_ERR_CUDA;
     nmsl_class_kernel<<<dim3(a.num_frames, kClassSlots), kClassThreads, smem_c, st>>>(a, ws, class_cap);
     TSCD_CUDA_CHECK_LAUNCH();
+    if (a.cand_cap > kNmsLargeCap) {
+        const int runs = (a.cand_cap + kRun - 1) / kRun;
+        const size_t smem_r = (size_t)kRun * 8;
+        if (cudaFuncSetAttribute(nmsw_run_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_r) != cudaSuccess) return TSCD_ERR_CUDA;
+        nmsw_run_kernel<<<dim3(a.num_frames, runs), kMergeThreads, smem_r, st>>>(a, ws);
+        TSCD_CUDA_CHECK_LAUNCH();
+        nmsw_rank_kernel<<<dim3(runs * kRun / 256, a.num_frames), 256, 0, st>>>(a, ws);
+        TSCD_CUDA_CHECK_LAUNCH();
+        nmsw_final_kernel<<<a.num_frames, kMergeThreads, 0, st>>>(a, ws);
+        TSCD_CUDA_CHECK_LAUNCH();
+        return TSCD_OK;
+    }
     int sort_cap = kMergeThreads;
     while (sort_cap < a.cand_cap) sort_cap <<= 1;
     const size_t smem_m = (size_t)sort_cap * (8 + 4);

@@ -11,8 +11,8 @@ from typing import List
 import torch
 
 from . import ops
-from .selection import SelectionConfig
-from .stage import AggregationStage, CAFMState, StageConfig, validate_config
+from .selection import DEFAULT_TIER_MAX, MAX_PROPOSALS, SelectionConfig
+from .stage import MAX_KEYS_PER_CLIP, AggregationStage, CAFMState, StageConfig, validate_config
 from .weights import timing_signal_1d  # noqa: F401  (re-exported for callers that build time embeddings)
 
 _CONV_PREFIXES = ("stems", "cls_convs", "reg_convs", "edge_enhance", "cls_preds", "reg_preds", "obj_preds")
@@ -27,9 +27,10 @@ def stage_config_from_head(head) -> StageConfig:
     if kw.get("local_mask", False) or head.use_mask or not head.ave:
         raise RuntimeError("TSCDHeadB200: local_mask / use_mask / ave=False are not implemented (not used by the TSCD exps)")
     # max_proposals: per-frame capacity of the proposal list.  The reference's list is unbounded when no maximal_limit is set
-    # (VID TSCD-L, exps/TSCD_VID/vid_tscd_large.py:39-42); the kernels hold at most 512 (fewer when 512 x classes would exceed
-    # the final NMS's 16384 candidate rows).  Overflow raises at forward time; kwargs['max_proposals'] overrides the default.
-    cap = min(512, ops.NMS_MAX_CAP // max(1, head.num_classes))
+    # (VID TSCD-L, exps/TSCD_VID/vid_tscd_large.py:39-42); the default tier holds at most 512 (fewer when 512 x classes would
+    # exceed the final NMS's 16384 candidate rows), and forward() reruns a call that overflows it on the wide tier
+    # (wide_capacity).  kwargs['max_proposals'] overrides the default and turns that escalation off: overflow then raises.
+    cap = min(DEFAULT_TIER_MAX, ops.NMS_MAX_CAP // max(1, head.num_classes))
     sel = SelectionConfig(mode="B", nms_thresh=head.nms_thresh, conf_thresh=0.001,
                           minimal_limit=kw.get("minimal_limit", 0), maximal_limit=kw.get("maximal_limit", 0),
                           use_pre_nms=kw.get("use_pre_nms", True), max_proposals=int(kw.get("max_proposals", cap)))
@@ -37,6 +38,12 @@ def stage_config_from_head(head) -> StageConfig:
                       conf_sim_thresh=kw.get("conf_sim_thresh", 0.99))
     validate_config(cfg)             # capacity problems surface when the head is built, not at the first forward
     return cfg
+
+
+def wide_capacity(num_frames: int, num_classes: int) -> int:
+    """Per-frame capacity of the wide tier for clips of `num_frames` frames: the attention kernels hold 65536 keys per clip and
+    the final NMS 65536 candidate rows (proposals x classes) per frame."""
+    return min(MAX_PROPOSALS, MAX_KEYS_PER_CLIP // max(1, num_frames), ops.NMS_WIDE_CAP // max(1, num_classes))
 
 
 def make_head_class():
@@ -49,6 +56,8 @@ def make_head_class():
             self._b200_stage = None
             self._b200_state = None
             self._b200_key = None
+            self._b200_wide = {}              # wide-tier stages by capacity (built on the first overflow)
+            self._b200_on_wide = False        # this video's resume=True calls stay on the wide tier
             stage_config_from_head(self)      # reject unsupported / over-capacity configurations at construction
             # model.load_state_dict(ckpt) recurses through _load_from_state_dict and never calls a child's load_state_dict:
             # the post-hook fires for this module either way
@@ -58,6 +67,8 @@ def make_head_class():
             self._b200_stage = None           # weights changed / moved: rebuild the 16-bit device copies lazily
             self._b200_state = None
             self._b200_edge = None
+            self._b200_wide = {}
+            self._b200_on_wide = False
 
         def _apply(self, fn, *a, **k):        # .half() / .to() / .cuda() / .float()
             self._b200_invalidate()
@@ -73,7 +84,20 @@ def make_head_class():
                 self._b200_stage = AggregationStage(stage_config_from_head(self), sd, device=params[0].device)
                 self._b200_key = key
                 self._b200_state = None
+                self._b200_wide = {}
+                self._b200_on_wide = False
             return self._b200_stage
+
+        def _wide_stage(self, cap):
+            """Stage of the wide tier (same weights as _stage(), per-frame capacity `cap`)."""
+            if cap not in self._b200_wide:
+                st = self._b200_stage
+                cfg = stage_config_from_head(self)
+                cfg.selection.max_proposals = cap
+                validate_config(cfg)
+                sd = {k: v for k, v in self.state_dict().items() if not k.startswith(_CONV_PREFIXES)}
+                self._b200_wide[cap] = AggregationStage(cfg, sd, device=st.device)
+            return self._b200_wide[cap]
 
         def _edge_block(self, dtype):
             """16-bit copies of the per-level WaveletsHFBlock weights for the selected-anchor evaluation (ops.EdgeBlock)."""
@@ -130,15 +154,37 @@ def make_head_class():
             st = self._stage()
             feats = (ops.view_levels(f_cls), ops.view_levels(f_reg),
                      ops.view_levels(f_edge) if dense_edge else self._edge_block(st.cfg.dtype))
-            st.cfg.final_nms_thresh = nms_thresh
             F = imgs.shape[0]
-            kmax = st.cfg.selection.max_keep(an.num_anchors)
-            if self._b200_state is None or self._b200_state.kmax != kmax:
+            # Tiers: a call runs on the default tier (<= 512 proposals per frame) unless the video is already on the wide tier.
+            # A default-tier call whose frames overflow is rerun on the wide tier from the CAFM memory it started with (the
+            # overflowing run may have written the memory), and the video's following resume=True calls stay there; the next
+            # resume=False call starts again on the default tier.  An explicit kwargs['max_proposals'] never escalates.
+            wide_cap = wide_capacity(F, self.num_classes)
+            can_widen = "max_proposals" not in self.kwargs and self.kwargs.get("maximal_limit", 0) == 0 \
+                and wide_cap > st.cfg.selection.max_proposals
+            if not resume:
+                self._b200_on_wide = False
+            on_wide = self._b200_on_wide and can_widen
+            run = self._wide_stage(wide_cap) if on_wide else st
+            run.cfg.final_nms_thresh = nms_thresh
+            kmax = run.cfg.selection.max_keep(an.num_anchors)
+            if self._b200_state is not None and resume and self._b200_state.kmax < kmax:
+                self._b200_state = self._b200_state.widened(kmax)
+            elif self._b200_state is None or self._b200_state.kmax != kmax:
                 self._b200_state = CAFMState(1, kmax, st.cfg.dim, imgs.device)
             res = torch.tensor([int(bool(resume))], dtype=torch.int32, device=imgs.device)
-            out = st.forward(head, feats, f_cls[0].dtype, time_embedding[:lframe].float(), 1, F, lframe,
-                             state=self._b200_state, resume=res)
-            result, result_ori = st.to_lists(out, 1, lframe)
+            te = time_embedding[:lframe].float()
+            snapshot = self._b200_state.flat.clone() if (resume and can_widen and not on_wide) else None
+            out = run.forward(head, feats, f_cls[0].dtype, te, 1, F, lframe, state=self._b200_state, resume=res)
+            if can_widen and not on_wide and int(out["status"].item()) != 0:
+                if snapshot is not None:
+                    self._b200_state.flat.copy_(snapshot)
+                run = self._wide_stage(wide_cap)
+                run.cfg.final_nms_thresh = nms_thresh
+                self._b200_state = self._b200_state.widened(run.cfg.selection.max_keep(an.num_anchors))
+                self._b200_on_wide = True
+                out = run.forward(head, feats, f_cls[0].dtype, te, 1, F, lframe, state=self._b200_state, resume=res)
+            result, result_ori = run.to_lists(out, 1, lframe)
             if int(out["sel"]["sel_count"].sum().item()) == 0:
                 # no proposal in any frame: the reference returns its F-length pred_result twice (tscd_head.py:439-440)
                 return [None] * F, [None] * F

@@ -242,17 +242,21 @@ def pred_heads(reg_feats: List[torch.Tensor], cls_feats: List[torch.Tensor], w_r
 
 
 NMS_SMEM_CAP = 4096       # csrc/nms.cuh kNmsCap: larger candidate lists take the workspace path (csrc/nms_large.cu)
-NMS_MAX_CAP = 16384       # kNmsLargeCap
+NMS_MAX_CAP = 16384       # kNmsLargeCap: per-frame merge in shared memory (the default tier's final-NMS limit)
+NMS_WIDE_CAP = 65536      # kNmsWideCap: merge through global memory (the wide tier's final-NMS limit)
 
 
 def nms(box: torch.Tensor, score: torch.Tensor, cls: torch.Tensor, count: torch.Tensor, iou_thresh: float,
         max_keep: Optional[int] = None, status: Optional[torch.Tensor] = None, strict_keep: bool = False, tag=None,
-        rank: Optional[torch.Tensor] = None):
+        rank: Optional[torch.Tensor] = None, wide: bool = False):
     """K2.  box [F,cap,4] f32, score [F,cap] f32, cls [F,cap] i32, count [F] i32 -> (keep [F,max_keep], keep_count [F]).
-    strict_keep: more than max_keep survivors in a frame is a capacity error (status) instead of a truncation."""
+    strict_keep: more than max_keep survivors in a frame is a capacity error (status) instead of a truncation.
+    wide: the caller is a wide-tier stage (SelectionConfig.max_proposals > 512) and accepts up to NMS_WIDE_CAP candidates per
+    frame (global-memory merge); otherwise the limit is NMS_MAX_CAP."""
     Fn, cap = score.shape
-    if cap > NMS_MAX_CAP:
-        raise RuntimeError(f"tscd_nms: {cap} candidates per frame exceed the kernel capacity of {NMS_MAX_CAP}")
+    limit = NMS_WIDE_CAP if wide else NMS_MAX_CAP
+    if cap > limit:
+        raise RuntimeError(f"tscd_nms: {cap} candidates per frame exceed the kernel capacity of {limit}")
     max_keep = cap if max_keep is None else max_keep
     keep = torch.empty(Fn, max_keep, dtype=torch.int32, device=score.device)
     keep_count = torch.empty(Fn, dtype=torch.int32, device=score.device)

@@ -20,6 +20,7 @@ import torch.distributed as dist
 
 from . import _lib as L
 from . import ops
+from .selection import DEFAULT_TIER_MAX
 
 
 def shard_clips(num_clips: int, rank: int, world: int):
@@ -97,6 +98,9 @@ def long_clip_forward(stage, sel, n_local_frames: int, n_global_frames: int, kma
     """Frame-sharded forward of ONE long clip.  `sel` = this rank's selection (frames ordered [local | global]);
     ranks hold consecutive blocks of the clip's local frames in rank order.  Returns the stage output for this rank's
     local frames (use AggregationStage.to_lists(out, 1, n_local_frames))."""
+    if kmax > DEFAULT_TIER_MAX:
+        raise RuntimeError(f"long_clip_forward: the long-clip mode supports the default tier only (<= {DEFAULT_TIER_MAX} "
+                           f"proposals per frame), got {kmax}")
     rank, world = dist.get_rank(group), dist.get_world_size(group)
     virt, F_virt = exchange_global_bank(sel, n_local_frames, n_global_frames, kmax, stage.cfg.dtype, group)
     dev = virt["bank_cls"].device

@@ -10,6 +10,14 @@ import torch
 
 from . import ops
 
+DEFAULT_TIER_MAX = 512     # max_proposals up to here: the default tier (csrc/cafm.cu kChainMax; 16384-row final NMS)
+MAX_PROPOSALS = 2048       # wide tier limit (include/tscd_b200.h TSCD_MAX_PROPOSALS)
+
+
+def is_wide(max_proposals: int) -> bool:
+    """Wide tier: more than DEFAULT_TIER_MAX proposals per frame (CTA LSAP, global-memory final-NMS merge)."""
+    return max_proposals > DEFAULT_TIER_MAX
+
 
 @dataclass
 class SelectionConfig:
@@ -25,9 +33,10 @@ class SelectionConfig:
     # conf_thresh: the reference's per-frame list is unbounded (up to all A = 6804 anchors), the kernels' buffers are not.
     # max_proposals is the explicit per-frame capacity of the proposal list (bank pitch, CAFM state / cost tables);
     # a frame that would keep more sets the stage's status flag and forward raises -- never a silent truncation.
-    max_proposals: int = 512        # the whole stage needs <= 512 (CAFM chain capacity, csrc/cafm.cu kChainMax); K1-K3 alone do not
+    # up to 512: the default tier; 513 .. MAX_PROPOSALS (2048): the wide tier (stage.validate_config states its limits)
+    max_proposals: int = 512
 
-    def validate(self, chain_capacity: int = 512):
+    def validate(self, chain_capacity: int = MAX_PROPOSALS):
         if self.mode not in ("A", "B"):
             raise RuntimeError(f"selection mode {self.mode!r}: expected 'A' (postpro_woclass) or 'B' (postprocess_widx)")
         if not 1 <= self.max_proposals <= chain_capacity:

@@ -44,7 +44,13 @@ def validate_config(cfg: StageConfig):
     kmax = sel.top_k if sel.mode == "A" else sel.max_proposals
     if sel.mode == "B" and sel.maximal_limit:
         kmax = max(sel.maximal_limit, sel.minimal_limit)
-    if kmax * cfg.num_classes > ops.NMS_MAX_CAP:
+    if _selection.is_wide(sel.max_proposals):
+        if kmax * cfg.num_classes > ops.NMS_WIDE_CAP:
+            raise RuntimeError(
+                f"final per-class NMS (wide tier, max_proposals = {sel.max_proposals} > {_selection.DEFAULT_TIER_MAX}): up to {kmax} "
+                f"proposals x {cfg.num_classes} classes = {kmax * cfg.num_classes} candidate rows per frame exceed the NMS capacity "
+                f"of {ops.NMS_WIDE_CAP}; lower max_proposals / maximal_limit to <= {ops.NMS_WIDE_CAP // cfg.num_classes}")
+    elif kmax * cfg.num_classes > ops.NMS_MAX_CAP:
         raise RuntimeError(
             f"final per-class NMS: up to {kmax} proposals x {cfg.num_classes} classes = {kmax * cfg.num_classes} candidate rows per "
             f"frame (post_process.py:36-46) exceed the NMS capacity of {ops.NMS_MAX_CAP}; lower max_proposals / maximal_limit "
@@ -96,6 +102,20 @@ class CAFMState:
     """Caller-owned CAFM memory (tscd_matching.py:708-715) for `slots` concurrent video streams.  All fields are views of ONE
     flat fp32 buffer (`flat`; `n` is its first `slots` words viewed as int32), so handing the memory to another rank in the
     long-clip mode is a single message."""
+
+    def widened(self, kmax: int) -> "CAFMState":
+        """Copy of this state with a larger row capacity `kmax` (rows beyond the old capacity are zero; the chain only reads
+        the first n).  The drop-in head moves a video's memory to the wide tier with it."""
+        if kmax < self.kmax:
+            raise RuntimeError(f"CAFMState.widened: kmax {kmax} < current {self.kmax}")
+        big = CAFMState(self.slots, kmax, self.dim, self.flat.device)
+        for f in self._FIELDS:
+            src, dst = getattr(self, f), getattr(big, f)
+            if f in ("n", "time"):
+                dst.copy_(src)
+            else:
+                dst[:, :self.kmax].copy_(src)
+        return big
 
     def __init__(self, slots: int, kmax: int, dim: int = 256, device="cuda"):
         self.slots, self.kmax, self.dim = slots, kmax, dim
@@ -234,6 +254,9 @@ class AggregationStage:
                             strides=(8, 16, 32), zero_copy_logits: bool = False, graph: bool = True, lanes: int = 4, slot: int = 0):
         """Launches one forward_host call without waiting for it; returns the ticket for forward_host_collect.  Calls submitted with
         different `slot`s own separate buffers and may be in flight together; a slot must be collected before it is reused."""
+        if _selection.is_wide(self.cfg.selection.max_proposals):
+            raise RuntimeError(f"forward_host: the host-buffer path supports the default tier only (max_proposals <= "
+                               f"{_selection.DEFAULT_TIER_MAX}); use forward() for max_proposals = {self.cfg.selection.max_proposals}")
         fused = "rows" in host
         head_keys = ("rows", "objp") if fused else ("reg", "obj", "cls")
         for k in head_keys + ("f_cls", "f_reg", "f_edge"):
@@ -605,7 +628,7 @@ class AggregationStage:
         out = {}
         for name, c, cap in (("det", r, rcap), ("ori", o, ocap)):
             keep, kc, _ = ops.nms(c["box"], c["score"], c["cls"], c["count"], cfg.final_nms_thresh, max_keep=cap, status=status,
-                                  tag="final_" + name)
+                                  tag="final_" + name, wide=_selection.is_wide(cfg.selection.max_proposals))
             rows = f32z(nlf, cap, 7)
             ops.call("tscd_final_rows", L.FinalRowsArgs, num_frames=nlf, cand_cap=cap, keep_cap=cap, box=c["box"],
                      obj=c["obj"], cscore=c["cscore"], cls=c["cls"], keep=keep, keep_count=kc, rows=rows)
@@ -731,7 +754,8 @@ class AggregationStage:
         st = int(out["status"].item())
         if st != 0:
             raise RuntimeError(f"tscd_b200 stage reported error {st} (capacity exceeded: a frame holds more proposals than "
-                               "SelectionConfig.max_proposals -- raise it (<= 512) or set maximal_limit)")
+                               f"the per-frame capacity of {out['sel']['sel_rows'].shape[1]} -- raise SelectionConfig.max_proposals "
+                               f"(<= {_selection.MAX_PROPOSALS}) or set maximal_limit)")
         det_n, ori_n = out["det_count"].cpu().tolist(), out["ori_count"].cpu().tolist()
         det_c = out["det_cand"].cpu().tolist()
         result, result_ori = [], []
