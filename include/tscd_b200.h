@@ -428,6 +428,9 @@ typedef struct {
     const void* emb_reg16;
     const void* emb_cls16;
     int32_t emb16_dtype;         /* TSCD_F16 / TSCD_BF16 */
+    /* optional state slot map: clip b reads the carried state (st_*) of slot slot[b] instead of slot b.  resume, lrow_off and
+     * the outputs stay indexed by the batch position b.  NULL = slot b (the state then holds exactly B slots). */
+    const int32_t* slot;         /* [B] */
 } tscd_cafm_cost_args;
 int tscd_cafm_cost(const tscd_cafm_cost_args* args, void* stream);
 
@@ -478,7 +481,7 @@ typedef struct {
     const float* ln_b;
     const float* dec_w;          /* decoder_norm */
     const float* dec_b;
-    /* state, caller-owned, persists across calls */
+    /* state, caller-owned, persists across calls; [B, ...] below reads [slots, ...] when `slot` is set */
     int32_t* st_n;               /* [B] rows held (0 = no memory) */
     float* st_out;               /* [B,kmax,D] */
     float* st_edge;              /* [B,kmax,D] */
@@ -500,6 +503,11 @@ typedef struct {
     int32_t* perm;               /* [loc_cap] matched column of every output row (debug / tests; may be NULL) */
     int32_t* status;
     int32_t emb_dtype;           /* element type of emb_reg / emb_cls: TSCD_F32 (0), or 16-bit with the fast path (widened into the state) */
+    /* optional state slot map: clip b reads and writes the state (st_*) of slot slot[b] instead of slot b, so a caller-owned
+     * state may hold more slots than the batch (one per concurrent video stream) and a call runs any B distinct slots of it
+     * without copies.  resume, the bank, the layout, the scratch and the outputs stay indexed by the batch position b.  The
+     * slots of one call must be distinct.  NULL = slot b.  tscd_cafm_wide reads it through `base`. */
+    const int32_t* slot;         /* [B] */
 } tscd_cafm_chain_args;
 int tscd_cafm_chain(const tscd_cafm_chain_args* args, void* stream);
 

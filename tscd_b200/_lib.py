@@ -126,7 +126,7 @@ class CafmChainArgs(C.Structure):
     _fields_ = _fields("B:i F:i L:i D:i kmax:i out_dtype:i row_off:p lrow_off:p resume:p feat:p edge:p kin:p kproj:p "
                        "vproj:p kproj16:p vproj16:p wq16:p bank_reg:p bank_edge:p time_emb:p emb_reg:p emb_cls:p norm_reg:p norm_cls:p wq_t:p se_w1:p se_w2:p ln_w:p "
                        "ln_b:p dec_w:p dec_b:p st_n:p st_out:p st_edge:p st_reg:p st_cls:p st_nreg:p st_ncls:p "
-                       "st_time:p sc_qin:p sc_q:p sc_k:p ref_n:p lap_col:p lap_row:p out16:p out32:p perm:p status:p emb_dtype:i")
+                       "st_time:p sc_qin:p sc_q:p sc_k:p ref_n:p lap_col:p lap_row:p out16:p out32:p perm:p status:p emb_dtype:i slot:p")
 
 
 class CafmWideArgs(C.Structure):
@@ -152,7 +152,7 @@ class EdgeCombineArgs(C.Structure):
 
 class CafmCostArgs(C.Structure):
     _fields_ = _fields("B:i L:i D:i kmax:i lrow_off:p resume:p st_n:p emb_reg:p emb_cls:p norm_reg:p norm_cls:p "
-                       "st_reg:p st_cls:p st_nreg:p st_ncls:p cost:p ref_n:p emb_dtype:i emb_reg16:p emb_cls16:p emb16_dtype:i")
+                       "st_reg:p st_cls:p st_nreg:p st_ncls:p cost:p ref_n:p emb_dtype:i emb_reg16:p emb_cls16:p emb16_dtype:i slot:p")
 
 
 class CafmLapArgs(C.Structure):

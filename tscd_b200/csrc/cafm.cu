@@ -175,11 +175,12 @@ __global__ void __launch_bounds__(kCwThreads) cafm_cost_wide16_kernel(const tscd
         }
     }
     if (np == 0) {
-        const int sn = (a.resume && a.resume[b]) ? a.st_n[b] : 0;
+        const int sb = a.slot ? a.slot[b] : b;       // state slot of clip b
+        const int sn = (a.resume && a.resume[b]) ? a.st_n[sb] : 0;
         if (sn > 0) {
             np = sn;
-            sR = a.st_reg + (int64_t)b * KM * E; sC = a.st_cls + (int64_t)b * KM * E;
-            nRp = a.st_nreg + (int64_t)b * KM; nCp = a.st_ncls + (int64_t)b * KM;
+            sR = a.st_reg + (int64_t)sb * KM * E; sC = a.st_cls + (int64_t)sb * KM * E;
+            nRp = a.st_nreg + (int64_t)sb * KM; nCp = a.st_ncls + (int64_t)sb * KM;
         } else {
             np = n;
             Rp = reinterpret_cast<const T*>(a.emb_reg16) + (int64_t)l0 * E; Cp = reinterpret_cast<const T*>(a.emb_cls16) + (int64_t)l0 * E;
@@ -310,11 +311,12 @@ __global__ void __launch_bounds__(256) cafm_cost_kernel(const tscd_cafm_cost_arg
         if (pn > 0) { np = pn; Rp = a.emb_reg + (int64_t)pl0 * E; Cp = a.emb_cls + (int64_t)pl0 * E; nRp = a.norm_reg + pl0; nCp = a.norm_cls + pl0; }
     }
     if (np == 0) {
-        const int sn = (a.resume && a.resume[b]) ? a.st_n[b] : 0;
+        const int sb = a.slot ? a.slot[b] : b;       // state slot of clip b
+        const int sn = (a.resume && a.resume[b]) ? a.st_n[sb] : 0;
         if (sn > 0) {
             np = sn;
-            Rp = a.st_reg + (int64_t)b * KM * E; Cp = a.st_cls + (int64_t)b * KM * E;
-            nRp = a.st_nreg + (int64_t)b * KM; nCp = a.st_ncls + (int64_t)b * KM;
+            Rp = a.st_reg + (int64_t)sb * KM * E; Cp = a.st_cls + (int64_t)sb * KM * E;
+            nRp = a.st_nreg + (int64_t)sb * KM; nCp = a.st_ncls + (int64_t)sb * KM;
         } else {
             np = n;
             Rp = a.emb_reg + (int64_t)l0 * E; Cp = a.emb_cls + (int64_t)l0 * E; nRp = a.norm_reg + l0; nCp = a.norm_cls + l0;
@@ -446,8 +448,9 @@ __global__ void __launch_bounds__(128) cafm_cost16_kernel(const tscd_cafm_cost_a
         if (pn > 0) { np = pn; Rp = reinterpret_cast<const T*>(a.emb_reg) + (int64_t)pl0 * E; Cp = reinterpret_cast<const T*>(a.emb_cls) + (int64_t)pl0 * E; }
     }
     if (np == 0) {
-        const int sn = (a.resume && a.resume[b]) ? a.st_n[b] : 0;
-        if (sn > 0) { np = sn; sR = a.st_reg + (int64_t)b * KM * E; sC = a.st_cls + (int64_t)b * KM * E; }
+        const int sb = a.slot ? a.slot[b] : b;       // state slot of clip b
+        const int sn = (a.resume && a.resume[b]) ? a.st_n[sb] : 0;
+        if (sn > 0) { np = sn; sR = a.st_reg + (int64_t)sb * KM * E; sC = a.st_cls + (int64_t)sb * KM * E; }
         else { np = n; Rp = reinterpret_cast<const T*>(a.emb_reg) + (int64_t)l0 * E; Cp = reinterpret_cast<const T*>(a.emb_cls) + (int64_t)l0 * E; }
     }
     if (np > KM || n > KM || np > 32 || n > 32) {          // the chain kernel reports the capacity error
@@ -903,20 +906,21 @@ __global__ void __launch_bounds__(kChainThreads, 1) cafm_chain_kernel(const tscd
     extern __shared__ __align__(16) unsigned char chain_smem[];
     ChainSmem& s = *reinterpret_cast<ChainSmem*>(chain_smem);
     const int b = blockIdx.x;
+    const int sb = a.slot ? a.slot[b] : b;   // state slot of clip b (scratch, bank and resume stay indexed by b)
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int D = a.D, E = 4 * a.D, KM = a.kmax;
     constexpr int NW = kChainThreads / 32;
     if (tid < 64) { s.w1[tid] = a.se_w1[tid]; s.w2[tid] = a.se_w2[tid]; }
 
-    float* st_out = a.st_out + (int64_t)b * KM * D;
-    float* st_edge = a.st_edge + (int64_t)b * KM * D;
-    float* st_time = a.st_time + (int64_t)b * D;
+    float* st_out = a.st_out + (int64_t)sb * KM * D;
+    float* st_edge = a.st_edge + (int64_t)sb * KM * D;
+    float* st_time = a.st_time + (int64_t)sb * D;
     float* g_qin = a.sc_qin + (int64_t)b * KM * D;
     float* g_q = a.sc_q + (int64_t)b * KM * D;
     float* g_k = a.sc_k + (int64_t)b * KM * D;
 
     const bool resume = a.resume ? (a.resume[b] != 0) : false;
-    int n_prev = resume ? a.st_n[b] : 0;   // 0 = no memory
+    int n_prev = resume ? a.st_n[sb] : 0;   // 0 = no memory
     for (int r = tid; r < kChainMax; r += kChainThreads) s.ord_prev[r] = r;   // carried state is already in matched order
     int last_l0 = -1;
     __syncthreads();
@@ -1071,8 +1075,8 @@ __global__ void __launch_bounds__(kChainThreads, 1) cafm_chain_kernel(const tscd
     }
     // ---- carry the last frame's matching embeddings (in matched order) to the next call ----------------
     if (last_l0 >= 0) {
-        float* st_reg = a.st_reg + (int64_t)b * KM * E;
-        float* st_cls = a.st_cls + (int64_t)b * KM * E;
+        float* st_reg = a.st_reg + (int64_t)sb * KM * E;
+        float* st_cls = a.st_cls + (int64_t)sb * KM * E;
         const float* Rc = a.emb_reg + (int64_t)last_l0 * E;
         const float* Cc = a.emb_cls + (int64_t)last_l0 * E;
         for (int t = tid; t < n_prev * (E / 4); t += kChainThreads) {
@@ -1082,11 +1086,11 @@ __global__ void __launch_bounds__(kChainThreads, 1) cafm_chain_kernel(const tscd
             reinterpret_cast<float4*>(st_cls)[(int64_t)r * (E / 4) + c4] = reinterpret_cast<const float4*>(Cc)[(int64_t)src * (E / 4) + c4];
         }
         for (int r = tid; r < n_prev; r += kChainThreads) {
-            a.st_nreg[(int64_t)b * KM + r] = a.norm_reg[last_l0 + s.ord_prev[r]];
-            a.st_ncls[(int64_t)b * KM + r] = a.norm_cls[last_l0 + s.ord_prev[r]];
+            a.st_nreg[(int64_t)sb * KM + r] = a.norm_reg[last_l0 + s.ord_prev[r]];
+            a.st_ncls[(int64_t)sb * KM + r] = a.norm_cls[last_l0 + s.ord_prev[r]];
         }
     }
-    if (tid == 0) a.st_n[b] = n_prev;
+    if (tid == 0) a.st_n[sb] = n_prev;
     __syncthreads();
     CHAIN_TICK(6);
 }
@@ -1180,7 +1184,7 @@ __global__ void __launch_bounds__(kFastThreads, 1) cafm_chain_fast_kernel(const 
         s.ln[0][c] = a.ln_w[c]; s.ln[1][c] = a.ln_b[c]; s.ln[2][c] = a.dec_w[c]; s.ln[3][c] = a.dec_b[c];
     }
     const bool resume = a.resume ? (a.resume[b] != 0) : false;
-    int n_prev = resume ? a.st_n[b] : 0;
+    int n_prev = resume ? a.st_n[a.slot ? a.slot[b] : b] : 0;
     bool bad = n_prev > kFR;
     int m = 0;                                   // number of non-empty frames (uniform: every thread scans the offsets)
     for (int f = 0; f < a.L; ++f) {
@@ -1210,13 +1214,14 @@ __global__ void __launch_bounds__(kFastThreads, 1) cafm_chain_fast_kernel(const 
     __syncthreads();                             // s.frames visible
     if (m > 0) fast_prefetch<T>(a, s.buf[0], b, s.frames[0], tid);
     if (n_prev > 0) {                            // resume: last_outputs -> x, last edge / time -> the "previous" buffer
-        const float* so = a.st_out + (int64_t)b * KM * 256;
-        const float* se = a.st_edge + (int64_t)b * KM * 256;
+        const int sb = a.slot ? a.slot[b] : b;   // state slot of clip b (re-read where needed: no register held across the loop)
+        const float* so = a.st_out + (int64_t)sb * KM * 256;
+        const float* se = a.st_edge + (int64_t)sb * KM * 256;
         for (int i = tid; i < n_prev * 256; i += kFastThreads) {
             s.x[i] = so[i];
             s.buf[1].edge[i] = cvt_from_float<T>(se[i]);          // exact: edge features are 16-bit bank values
         }
-        for (int c = tid; c < 256; c += kFastThreads) s.buf[1].time[c] = a.st_time[(int64_t)b * 256 + c];
+        for (int c = tid; c < 256; c += kFastThreads) s.buf[1].time[c] = a.st_time[(int64_t)sb * 256 + c];
     }
     int slot = 0, last_l0 = -1;
 
@@ -1444,18 +1449,19 @@ __global__ void __launch_bounds__(kFastThreads, 1) cafm_chain_fast_kernel(const 
     __syncthreads();
 
     // ---- write the memory back (tscd_matching.py:876-878) for the next call ------------------------------------
+    const int sb = a.slot ? a.slot[b] : b;
     if (last_l0 >= 0) {
         const FastBuf<T>& lastb = s.buf[slot ^ 1];
-        float* so = a.st_out + (int64_t)b * KM * 256;
-        float* se = a.st_edge + (int64_t)b * KM * 256;
+        float* so = a.st_out + (int64_t)sb * KM * 256;
+        float* se = a.st_edge + (int64_t)sb * KM * 256;
         for (int i = tid; i < n_prev * 256; i += kFastThreads) {
             const int r = i >> 8, c = i & 255;
             so[i] = s.x[i];
             se[i] = ldf_reg(lastb.edge[s.ord_prev[r] * 256 + c]);
         }
-        for (int c = tid; c < 256; c += kFastThreads) a.st_time[(int64_t)b * 256 + c] = lastb.time[c];
-        float* st_reg = a.st_reg + (int64_t)b * KM * E;
-        float* st_cls = a.st_cls + (int64_t)b * KM * E;
+        for (int c = tid; c < 256; c += kFastThreads) a.st_time[(int64_t)sb * 256 + c] = lastb.time[c];
+        float* st_reg = a.st_reg + (int64_t)sb * KM * E;
+        float* st_cls = a.st_cls + (int64_t)sb * KM * E;
         if (a.emb_dtype != TSCD_F32) {
             // 16-bit matching embeddings: widened to fp32 in the state (exact), 8 values per 16-byte load
             const T* Rc16 = reinterpret_cast<const T*>(a.emb_reg) + (int64_t)last_l0 * E;
@@ -1496,11 +1502,11 @@ __global__ void __launch_bounds__(kFastThreads, 1) cafm_chain_fast_kernel(const 
             }
         }
         for (int r = tid; r < n_prev; r += kFastThreads) {
-            a.st_nreg[(int64_t)b * KM + r] = a.norm_reg[last_l0 + s.ord_prev[r]];
-            a.st_ncls[(int64_t)b * KM + r] = a.norm_cls[last_l0 + s.ord_prev[r]];
+            a.st_nreg[(int64_t)sb * KM + r] = a.norm_reg[last_l0 + s.ord_prev[r]];
+            a.st_ncls[(int64_t)sb * KM + r] = a.norm_cls[last_l0 + s.ord_prev[r]];
         }
     }
-    if (tid == 0) a.st_n[b] = n_prev;
+    if (tid == 0) a.st_n[sb] = n_prev;
 }
 
 
@@ -1526,7 +1532,7 @@ __global__ void cafm_wide_begin_kernel(const tscd_cafm_wide_args w) {
     const int b = blockIdx.x, KM = a.kmax;
     const bool resume = a.resume ? (a.resume[b] != 0) : false;
     for (int r = threadIdx.x; r < KM; r += blockDim.x) w.ord_prev[(int64_t)b * KM + r] = r;
-    if (threadIdx.x == 0) { w.n_prev[b] = resume ? a.st_n[b] : 0; w.last_l0[b] = -1; }
+    if (threadIdx.x == 0) { w.n_prev[b] = resume ? a.st_n[a.slot ? a.slot[b] : b] : 0; w.last_l0[b] = -1; }
 }
 
 // one CTA (512 threads, rows in chunks of 512) per clip: control block + perm / prow of frame f (tscd_matching.py:813-844)
@@ -1596,9 +1602,10 @@ __global__ void __launch_bounds__(256) cafm_wide_qin_kernel(const tscd_cafm_wide
     if (threadIdx.x < 64) { w1[threadIdx.x] = a.se_w1[threadIdx.x]; w2[threadIdx.x] = a.se_w2[threadIdx.x]; }
     __syncthreads();
     T* qin = reinterpret_cast<T*>(w.qin16) + (int64_t)b * KM * D;
-    const float* st_out = a.st_out + (int64_t)b * KM * D;
-    const float* st_edge = a.st_edge + (int64_t)b * KM * D;
-    const float tm = a.st_time[(int64_t)b * D + c];
+    const int sb = a.slot ? a.slot[b] : b;           // state slot of clip b
+    const float* st_out = a.st_out + (int64_t)sb * KM * D;
+    const float* st_edge = a.st_edge + (int64_t)sb * KM * D;
+    const float tm = a.st_time[(int64_t)sb * D + c];
     const int* prow = w.prow_s + (int64_t)b * KM;
     for (int r = blockIdx.y * 8; r < min(KM, blockIdx.y * 8 + 8); ++r) {
         float v = 0.f;
@@ -1627,8 +1634,9 @@ __global__ void __launch_bounds__(256) cafm_wide_finish_kernel(const tscd_cafm_w
     const int lf = b * a.L + f, n = ctl.n, l0 = ctl.l0;
     const bool first = ctl.first != 0;
     const int* perm = w.perm_s + (int64_t)b * KM;
-    float* st_out = a.st_out + (int64_t)b * KM * D;
-    float* st_edge = a.st_edge + (int64_t)b * KM * D;
+    const int sb = a.slot ? a.slot[b] : b;           // state slot of clip b
+    float* st_out = a.st_out + (int64_t)sb * KM * D;
+    float* st_edge = a.st_edge + (int64_t)sb * KM * D;
     const int r = blockIdx.y * 8 + warp;
     if (r < n) {
         const int pr = perm[r];
@@ -1653,7 +1661,7 @@ __global__ void __launch_bounds__(256) cafm_wide_finish_kernel(const tscd_cafm_w
         }
     }
     if (blockIdx.y == 0) {
-        for (int c = threadIdx.x; c < D; c += blockDim.x) a.st_time[(int64_t)b * D + c] = a.time_emb[(int64_t)lf * D + c];
+        for (int c = threadIdx.x; c < D; c += blockDim.x) a.st_time[(int64_t)sb * D + c] = a.time_emb[(int64_t)lf * D + c];
         if (threadIdx.x == 0) { w.n_prev[b] = n; w.last_l0[b] = l0; }
     }
 }
@@ -1665,9 +1673,10 @@ __global__ void __launch_bounds__(256) cafm_wide_end_kernel(const tscd_cafm_wide
     const int nthreads = gridDim.y * blockDim.x;
     const int n_prev = w.n_prev[b], last_l0 = w.last_l0[b];
     const int* ord = w.ord_prev + (int64_t)b * KM;
+    const int sb = a.slot ? a.slot[b] : b;           // state slot of clip b
     if (last_l0 >= 0) {
-        float* st_reg = a.st_reg + (int64_t)b * KM * E;
-        float* st_cls = a.st_cls + (int64_t)b * KM * E;
+        float* st_reg = a.st_reg + (int64_t)sb * KM * E;
+        float* st_cls = a.st_cls + (int64_t)sb * KM * E;
         const float* Rc = a.emb_reg + (int64_t)last_l0 * E;
         const float* Cc = a.emb_cls + (int64_t)last_l0 * E;
         for (int t = tid; t < n_prev * (E / 4); t += nthreads) {
@@ -1677,11 +1686,11 @@ __global__ void __launch_bounds__(256) cafm_wide_end_kernel(const tscd_cafm_wide
             reinterpret_cast<float4*>(st_cls)[(int64_t)r * (E / 4) + c4] = reinterpret_cast<const float4*>(Cc)[(int64_t)src * (E / 4) + c4];
         }
         for (int r = tid; r < n_prev; r += nthreads) {
-            a.st_nreg[(int64_t)b * KM + r] = a.norm_reg[last_l0 + ord[r]];
-            a.st_ncls[(int64_t)b * KM + r] = a.norm_cls[last_l0 + ord[r]];
+            a.st_nreg[(int64_t)sb * KM + r] = a.norm_reg[last_l0 + ord[r]];
+            a.st_ncls[(int64_t)sb * KM + r] = a.norm_cls[last_l0 + ord[r]];
         }
     }
-    if (tid == 0) a.st_n[b] = n_prev;
+    if (tid == 0) a.st_n[sb] = n_prev;
 }
 
 }  // namespace tscd

@@ -62,6 +62,46 @@ def validate_config(cfg: StageConfig):
 MAX_KEYS_PER_CLIP = 65536     # attention kernels: keys of one clip (csrc/attn.cu, 16-bit key index in row_meta)
 
 
+def check_state_args(B: int, kmax: int, state=None, resume=None, state_slots=None, host: bool = False):
+    """Validates the CAFM-memory arguments of one call of B clips (no device work; raises RuntimeError).
+
+    state: a CAFMState; resume: [B] flags; state_slots: [B] slot of every clip in `state` (a list / array, or an int32 device
+    tensor, whose values are then not read back: capture-safe).  Without state_slots the state holds exactly B slots (clip b
+    uses slot b).  host=True: the forward_host rules -- state, resume and state_slots go together.  host=False: the device
+    path, which refuses a pool that still has forward_host calls in flight (their CAFM phases are ordered on the device
+    only among themselves)."""
+    where = "forward_host" if host else "forward"
+    if state is None:
+        if state_slots is not None or (host and resume is not None):
+            raise RuntimeError(f"{where}: resume / state_slots were given without state; pass the CAFMState pool they refer to")
+        return
+    if host and (resume is None or state_slots is None):
+        raise RuntimeError(f"{where}: state needs resume and state_slots (one resume flag and one state slot per clip)")
+    if state.kmax != kmax:
+        raise RuntimeError(f"{where}: the CAFMState holds {state.kmax} rows per slot, this configuration needs kmax = {kmax} "
+                           f"(SelectionConfig.max_keep); allocate CAFMState(slots, {kmax})")
+    for name, v in (("resume", resume), ("state_slots", state_slots)):
+        if host and isinstance(v, torch.Tensor) and v.device.type != "cpu":
+            raise RuntimeError(f"{where}: {name} must be host-side (a list, NumPy array or CPU tensor); it is copied with the call")
+        if v is not None and len(v) != B:
+            raise RuntimeError(f"{where}: {name} has {len(v)} entries for {B} clips")
+    if state_slots is not None:
+        if isinstance(state_slots, torch.Tensor) and state_slots.is_cuda:
+            if state_slots.dtype != torch.int32 or state_slots.dim() != 1:
+                raise RuntimeError(f"{where}: a device state_slots tensor must be 1-D int32")
+        else:
+            sl = np.asarray(state_slots.cpu() if isinstance(state_slots, torch.Tensor) else state_slots).reshape(-1)
+            bad = [int(x) for x in sl if not 0 <= int(x) < state.slots]
+            if bad:
+                raise RuntimeError(f"{where}: state slot(s) {bad} outside [0, {state.slots}) of the CAFMState pool")
+            if len(set(int(x) for x in sl)) != len(sl):
+                raise RuntimeError(f"{where}: duplicate state slot in one call ({sorted(int(x) for x in sl)}); the clips of a "
+                                   "call run concurrently and need distinct slots")
+    if not host and state._host_in_flight:
+        raise RuntimeError(f"{where}: the CAFMState pool still has {state._host_in_flight} forward_host call(s) in flight; "
+                           "collect them (forward_host_collect) before using the pool on the device path")
+
+
 class StageWeights:
     """Device copies of the aggregation-stage parameters (reference state_dict key names, SURVEY App. B)."""
 
@@ -119,6 +159,9 @@ class CAFMState:
 
     def __init__(self, slots: int, kmax: int, dim: int = 256, device="cuda"):
         self.slots, self.kmax, self.dim = slots, kmax, dim
+        self._host_in_flight = 0           # submitted, not yet collected stateful forward_host calls on this pool
+        self._host_cafm_done = None        # CAFM-done event of the most recently submitted of them (ordering of pool accesses)
+        self._host_order_stream = None     # stream on which those calls' gates are recorded (created by the first of them)
         sizes = [("n", slots), ("out", slots * kmax * dim), ("edge", slots * kmax * dim), ("reg", slots * kmax * 4 * dim),
                  ("cls", slots * kmax * 4 * dim), ("nreg", slots * kmax), ("ncls", slots * kmax), ("time", slots * dim)]
         total = sum(((n + 3) // 4) * 4 for _, n in sizes)            # every field 16-byte aligned
@@ -203,7 +246,11 @@ class AggregationStage:
 
     # ------------------------------------------------------------------------------------------------------
     def forward(self, head: ops.HeadViews, feats, feat_dtype, time_embedding: torch.Tensor, B: int, F: int, Lf: int,
-                state: Optional[CAFMState] = None, resume: Optional[torch.Tensor] = None, trace: Optional[dict] = None):
+                state: Optional[CAFMState] = None, resume: Optional[torch.Tensor] = None, trace: Optional[dict] = None,
+                state_slots=None):
+        """state_slots (optional, with `state`): [B] slot of every clip in `state` (list, or int32 device tensor -- the latter
+        under CUDA-graph capture); the kernels then read and write those slots in place, so `state` may be a pool with more
+        slots than clips (one per concurrent video).  Without it `state` holds exactly B slots, clip b in slot b."""
         cfg, w, dev, dt = self.cfg, self.w, self.device, self.cfg.dtype
         C = cfg.num_classes
         D = cfg.dim
@@ -213,6 +260,7 @@ class AggregationStage:
         if _r128(F * kmax) > MAX_KEYS_PER_CLIP:
             raise RuntimeError(f"{F} frames x {kmax} proposals per frame = {F * kmax} keys per clip exceed the attention kernels' "
                                f"capacity of {MAX_KEYS_PER_CLIP}; lower SelectionConfig.max_proposals")
+        check_state_args(B, kmax, state, resume, state_slots)
         status = torch.zeros(1, dtype=torch.int32, device=dev)
 
         # ---- K1-K3: selection + bank (operand arrays are read in 128-row TMA boxes: capacity padded) ------
@@ -220,11 +268,12 @@ class AggregationStage:
         sel = _selection.select_and_gather(head, feats, feat_dtype, D, cfg.selection, bank_dtype=dt, status=status,
                                            bank_rows=row_cap)
         return self.forward_from_bank(sel, B, F, Lf, kmax, time_embedding, state=state, resume=resume, trace=trace,
-                                      status=status)
+                                      status=status, state_slots=state_slots)
 
     # ------------------------------------------------------------------------------------------------------
     def forward_host(self, host: dict, hw, time_embedding: torch.Tensor, B: int, F: int, Lf: int, chunk_clips: int = 8,
-                     strides=(8, 16, 32), zero_copy_logits: bool = False, graph: bool = True, lanes: int = 4):
+                     strides=(8, 16, 32), zero_copy_logits: bool = False, graph: bool = True, lanes: int = 4,
+                     state: Optional[CAFMState] = None, resume=None, state_slots=None):
         """The stage for callers whose boundary tensors live in (pinned) HOST memory -> detections on the host.
 
         `host` holds per-level lists of pinned CPU tensors: the feature planes f_cls, f_reg, f_edge ([B*F, 256, H, W],
@@ -246,17 +295,29 @@ class AggregationStage:
         forward_host = forward_host_submit + forward_host_collect; callers that stream clips keep two calls in flight (two
         `slot`s: separate staging / output buffers and graphs) so that the PCIe phases of one call overlap the compute tail and the
         host-side unpacking of the previous one.
+        CAFM memory: without `state` every clip starts a new video (resume 0; the plan's own scratch memory).  With `state` (a
+        caller-owned CAFMState pool of any number of slots >= B, kmax = SelectionConfig.max_keep), `resume` ([B] flags) and
+        `state_slots` ([B] distinct slots of the pool) the call continues the videos held in those slots, exactly like
+        forward(state=, resume=, state_slots=): a video's clips can be streamed through successive calls.  The flags and the
+        slot map are copied per call, so one captured plan serves every slot map.
         Returns (result, result_ori, h2d_bytes, d2h_bytes) with fresh host tensors in the reference's list layout."""
         return self.forward_host_collect(self.forward_host_submit(host, hw, time_embedding, B, F, Lf, chunk_clips, strides,
-                                                                  zero_copy_logits, graph, lanes))
+                                                                  zero_copy_logits, graph, lanes, state=state, resume=resume,
+                                                                  state_slots=state_slots))
 
     def forward_host_submit(self, host: dict, hw, time_embedding: torch.Tensor, B: int, F: int, Lf: int, chunk_clips: int = 8,
-                            strides=(8, 16, 32), zero_copy_logits: bool = False, graph: bool = True, lanes: int = 4, slot: int = 0):
+                            strides=(8, 16, 32), zero_copy_logits: bool = False, graph: bool = True, lanes: int = 4, slot: int = 0,
+                            state: Optional[CAFMState] = None, resume=None, state_slots=None):
         """Launches one forward_host call without waiting for it; returns the ticket for forward_host_collect.  Calls submitted with
-        different `slot`s own separate buffers and may be in flight together; a slot must be collected before it is reused."""
+        different `slot`s own separate buffers and may be in flight together; a slot must be collected before it is reused.
+        (`slot` is the in-flight buffer set; `state_slots` are CAFM memory slots of `state`, see forward_host.)
+        Stateful calls on one pool access it in submission order: each call's CAFM phases (matching costs + chain) wait for
+        those of the call submitted before it on the same pool, while its copies, selection and attention overlap them."""
         if _selection.is_wide(self.cfg.selection.max_proposals):
             raise RuntimeError(f"forward_host: the host-buffer path supports the default tier only (max_proposals <= "
                                f"{_selection.DEFAULT_TIER_MAX}); use forward() for max_proposals = {self.cfg.selection.max_proposals}")
+        check_state_args(B, self.cfg.selection.max_keep(ops.AnchorSpec(hw, strides).num_anchors), state, resume, state_slots,
+                         host=True)
         fused = "rows" in host
         head_keys = ("rows", "objp") if fused else ("reg", "obj", "cls")
         for k in head_keys + ("f_cls", "f_reg", "f_edge"):
@@ -266,11 +327,13 @@ class AggregationStage:
                                        "read them in place; there is no pageable-memory / CPU path")
         key = (tuple((k, t.data_ptr(), tuple(t.shape), t.stride(), t.dtype) for k in head_keys + ("f_cls", "f_reg", "f_edge") for t in host[k]),
                tuple(tuple(x) for x in hw), tuple(strides), B, F, Lf, chunk_clips, zero_copy_logits, graph, lanes,
-               tuple(time_embedding.shape), slot)
+               tuple(time_embedding.shape), slot,
+               None if state is None else (state.flat.data_ptr(), state.slots, state.kmax, state.dim))   # the graph holds the pool's field pointers
         plans = self.__dict__.setdefault("_host_plans", {})
         plan = plans.pop(key, None)
         if plan is None:
-            plan = self._build_host_plan(host, hw, time_embedding, B, F, Lf, chunk_clips, strides, zero_copy_logits, graph, fused, lanes)
+            plan = self._build_host_plan(host, hw, time_embedding, B, F, Lf, chunk_clips, strides, zero_copy_logits, graph, fused, lanes,
+                                         state)
             self.host_plan_builds = getattr(self, "host_plan_builds", 0) + 1      # diagnostics: a caller that keeps missing the plan cache pays a capture per call
         plans[key] = plan                                      # most recently used last
         while len(plans) > 8:
@@ -284,14 +347,30 @@ class AggregationStage:
         # spinning) the whole intra-op pool once per call starves this thread on CPU-quota-limited containers (measured: 8 ms here
         # and 28 ms in the unpack instead of 0.2 / 0.5 ms, intermittently, depending on the box)
         np.copyto(plan["te_pin"].numpy(), time_embedding.detach().cpu().numpy())
+        if state is not None:
+            np.copyto(plan["resume_pin"].numpy(), np.asarray(resume, dtype=np.int64).reshape(-1), casting="unsafe")
+            np.copyto(plan["slots_pin"].numpy(), np.asarray(state_slots, dtype=np.int64).reshape(-1), casting="unsafe")
+            # ordering of the pool's accesses: this call's CAFM phases (graph: event-wait nodes on `gate`) start after the
+            # previous call's on the same pool have finished (its `cafm_done`).  One ordering stream per pool: calls on other
+            # pools do not wait for this one.
+            if state._host_order_stream is None:
+                state._host_order_stream = torch.cuda.Stream(device=self.device)
+            order = state._host_order_stream
+            if state._host_cafm_done is not None:
+                order.wait_event(state._host_cafm_done)
+            plan["gate"].record(order)
         if plan["graph"] is not None:
             with torch.cuda.stream(plan["launch"]):            # one launch stream per plan: calls of different slots run concurrently
                 plan["graph"].replay()
                 plan["done"].record()
         else:
-            plan["issue"]()
+            plan["issue"](state)
             plan["done"].record()
+        if state is not None:                                  # launched: from here on this call is the pool's last one
+            state._host_cafm_done = plan["cafm_done"]
+            state._host_in_flight += 1
         plan["busy"] = True
+        plan["pool"] = state
         return plan
 
     def forward_host_collect(self, plan, timing: Optional[dict] = None):
@@ -302,6 +381,9 @@ class AggregationStage:
         plan["done"].synchronize()
         t1 = _time.perf_counter()
         plan["busy"] = False
+        if plan.get("pool") is not None:
+            plan["pool"]._host_in_flight -= 1
+            plan["pool"] = None
         result, result_ori, d2h = [], [], 0
         h2d = plan["h2d"]
         for nc, pk in plan["pend"]:
@@ -315,8 +397,10 @@ class AggregationStage:
             timing["unpack"] = 1e3 * (_time.perf_counter() - t1)
         return result, result_ori, h2d, d2h
 
-    def _build_host_plan(self, host, hw, time_embedding, B, F, Lf, chunk_clips, strides, zero_copy_logits, graph, fused, n_lanes):
-        """Staging buffers + the launch sequence of one forward_host call (optionally captured into a CUDA graph)."""
+    def _build_host_plan(self, host, hw, time_embedding, B, F, Lf, chunk_clips, strides, zero_copy_logits, graph, fused, n_lanes,
+                         pool=None):
+        """Staging buffers + the launch sequence of one forward_host call (optionally captured into a CUDA graph).
+        pool: the caller's CAFMState (stateful plan) or None (the plan owns one scratch CAFMState per chunk: resume 0)."""
         dev = self.device
         an = ops.AnchorSpec(hw, strides)
         feat_dtype = host["f_cls"][0].dtype
@@ -340,14 +424,32 @@ class AggregationStage:
         plan = {"te_pin": te_pin, "graph": None, "pend": None, "h2d": 0, "_keep": (dbuf, host, cp, aux, io), "Lf": Lf, "busy": False,
                 "done": torch.cuda.Event(), "launch": torch.cuda.Stream(device=dev, priority=-1)}
         fused_row_bytes = host["rows"][0].shape[2] * 2 if fused else None
+        kmax = self.cfg.selection.max_keep(an.num_anchors)
+        if pool is None:
+            # stateless: CAFM memory owned by the plan, one state per chunk (chunks run concurrently); never read (resume 0)
+            plan["states"] = [CAFMState(nc, kmax, self.cfg.dim, dev) for _, nc in chunks]
+        else:
+            # stateful: per-call resume flags and slot map, filled by forward_host_submit and copied with the call; external
+            # events so that the ordering also holds between graph replays (event record / wait nodes)
+            plan["resume_pin"] = torch.zeros(B, dtype=torch.int32, pin_memory=True)
+            plan["slots_pin"] = torch.arange(B, dtype=torch.int32).pin_memory()
+            plan["gate"], plan["cafm_done"] = torch.cuda.Event(external=True), torch.cuda.Event(external=True)
+            plan["cafm_join"] = torch.cuda.Stream(device=dev)
+            plan["_keep"] += (pool,)          # the graph holds the pool's pointers: its memory must not go to another pool
+            for ev in (plan["gate"], plan["cafm_done"]):   # created (recorded once) before capture: waits on an unrecorded event are no-ops
+                ev.record(torch.cuda.current_stream())
 
-        def issue():
+        def issue(st=None):
             main = torch.cuda.current_stream()
             cp.wait_stream(main)                               # earlier work on this stream is done with the staging buffers
             events, h2d = [], 0
             with torch.cuda.stream(cp):
                 te_dev = te_pin.to(dev, non_blocking=True)
                 h2d += te_pin.numel() * te_pin.element_size()
+                if st is not None:
+                    resume_dev = plan["resume_pin"].to(dev, non_blocking=True)
+                    slots_dev = plan["slots_pin"].to(dev, non_blocking=True)
+                    h2d += 2 * 4 * B
                 for (c0, nc) in chunks:
                     f0, f1 = c0 * F, (c0 + nc) * F
                     for k in copied:
@@ -363,7 +465,6 @@ class AggregationStage:
             # while the tensor-core / latency-bound tail of the previous chunks runs on the compute lanes.  (Chunks that walk
             # through all phases in lockstep on parallel lanes leave the link idle during every compute phase.)
             cfg_sel = self.cfg.selection
-            kmax = cfg_sel.max_keep(an.num_anchors)
             if _r128(F * kmax) > MAX_KEYS_PER_CLIP:
                 raise RuntimeError(f"{F} frames x {kmax} proposals per frame exceed the attention kernels' capacity of {MAX_KEYS_PER_CLIP} keys per clip")
             lanes = ([main] + aux)[:max(1, min(len(chunks), n_lanes))]
@@ -389,16 +490,33 @@ class AggregationStage:
                     evb = torch.cuda.Event()
                     evb.record(io)
                     banks.append((sel, status, evb))
-            pend = []
+            pend, cafm_evs = [], []
             for ci, ((c0, nc), (sel, status, evb)) in enumerate(zip(chunks, banks)):
                 lane_s = lanes[ci % len(lanes)]
                 with torch.cuda.stream(lane_s):
                     lane_s.wait_event(evb)
                     if lane_s is not main:
-                        te_dev.record_stream(lane_s)
-                    out = self.forward_from_bank(sel, nc, F, Lf, kmax, te_dev[c0 * Lf:(c0 + nc) * Lf], status=status)
+                        for t in (te_dev,) if st is None else (te_dev, resume_dev, slots_dev):
+                            t.record_stream(lane_s)
+                    te_c = te_dev[c0 * Lf:(c0 + nc) * Lf]
+                    if st is None:
+                        out = self._from_bank(sel, nc, F, Lf, kmax, te_c, plan["states"][ci], None, status=status)
+                    else:                      # chunk c0..c0+nc: its slice of the flags and of the slot map
+                        ev_c = torch.cuda.Event()
+                        out = self._from_bank(sel, nc, F, Lf, kmax, te_c, st, resume_dev[c0:c0 + nc], status=status,
+                                              state_slots=slots_dev[c0:c0 + nc], cafm_gate=plan["gate"],
+                                              after_cafm=lambda _s, e=ev_c: e.record())
+                        cafm_evs.append(ev_c)
                     reuse = plan["pend"][len(pend)][1] if plan["pend"] is not None else None
                     pend.append((nc, self._pack_to_host(out, zc or rows_in_place, fused_row_bytes, reuse)))
+            if st is not None:                 # every chunk's chain is done with the pool -> the next call on it may start its CAFM
+                ordst = plan["cafm_join"]
+                for e in cafm_evs:
+                    ordst.wait_event(e)
+                plan["cafm_done"].record(ordst)
+                main.wait_stream(ordst)
+                for t in (resume_dev, slots_dev):
+                    t.record_stream(main)
             main.wait_stream(io)
             for a_ in lanes[1:]:
                 main.wait_stream(a_)
@@ -409,15 +527,17 @@ class AggregationStage:
         plan["issue"] = issue
         if graph:
             # warm up (lazy module loading, per-stream stage state) and capture on one high-priority stream, like capture_fn
+            # (a stateful plan warms up on a throwaway pool of the same shape -- resume_pin is still 0 -- so that the real pool is
+            # advanced by the replays only, and is captured against the real pool)
             hp = torch.cuda.Stream(device=dev, priority=-1)
             hp.wait_stream(torch.cuda.current_stream())
             with torch.cuda.stream(hp):
-                issue()
+                issue(None if pool is None else CAFMState(pool.slots, pool.kmax, pool.dim, dev))
             torch.cuda.current_stream().wait_stream(hp)
             torch.cuda.synchronize()
             g = torch.cuda.CUDAGraph()
             with torch.cuda.graph(g, stream=hp):
-                issue()
+                issue(pool)
             plan["graph"] = g
         return plan
 
@@ -476,27 +596,33 @@ class AggregationStage:
 
     # ------------------------------------------------------------------------------------------------------
     def capture(self, head: ops.HeadViews, feats, feat_dtype, time_embedding: torch.Tensor, B: int, F: int, Lf: int,
-                state: Optional["CAFMState"] = None, resume: Optional[torch.Tensor] = None, warmup: int = 2):
+                state: Optional["CAFMState"] = None, resume: Optional[torch.Tensor] = None, warmup: int = 2, state_slots=None):
         """Capture one forward() over FIXED input buffers into a CUDA graph (the stage has no host sync, so the whole
         launch sequence -- ~130 kernels on two streams -- replays from one cudaGraphLaunch).  Returns (graph, out):
-        refill the input tensors in place, call graph.replay(), read `out` (same dict forward() returns)."""
+        refill the input tensors in place, call graph.replay(), read `out` (same dict forward() returns).
+        state_slots: as in forward(); a list is copied to a device tensor once, refill that (out["state_slots"]) to remap."""
         A = head.anchors.num_anchors
         kmax = self.cfg.selection.max_keep(A)
+        check_state_args(B, kmax, state, resume, state_slots)
         if state is None:
             state = CAFMState(B, kmax, self.cfg.dim, self.device)
         if resume is None:
             resume = torch.zeros(B, dtype=torch.int32, device=self.device)
+        if state_slots is not None and not (isinstance(state_slots, torch.Tensor) and state_slots.is_cuda):
+            state_slots = torch.tensor([int(x) for x in state_slots], dtype=torch.int32, device=self.device)
         te = time_embedding.to(self.device)
         s = torch.cuda.Stream(device=self.device)
         s.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(s):                     # warm-up on a side stream (lazy module loading, attribute setting)
             for _ in range(warmup):
-                self.forward(head, feats, feat_dtype, te, B, F, Lf, state=state, resume=resume)
+                self.forward(head, feats, feat_dtype, te, B, F, Lf, state=state, resume=resume, state_slots=state_slots)
         torch.cuda.current_stream().wait_stream(s)
         torch.cuda.synchronize()
         graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(graph):
-            out = self.forward(head, feats, feat_dtype, te, B, F, Lf, state=state, resume=resume)
+            out = self.forward(head, feats, feat_dtype, te, B, F, Lf, state=state, resume=resume, state_slots=state_slots)
+        if state_slots is not None:
+            out["state_slots"] = state_slots
         return graph, out
 
     # ------------------------------------------------------------------------------------------------------
@@ -521,10 +647,18 @@ class AggregationStage:
 
     # ------------------------------------------------------------------------------------------------------
     def forward_from_bank(self, sel, B: int, F: int, Lf: int, kmax: int, time_embedding, state=None, resume=None,
-                          trace=None, status=None, before_cafm=None, after_cafm=None):
+                          trace=None, status=None, before_cafm=None, after_cafm=None, state_slots=None):
         """Everything after K1-K3.  `sel` holds the packed clip bank (bank_cls/reg/edge/score with >= _r128(B*F*kmax)+128
         rows), sel_count [B*F], row_off [B*F+1] and sel_rows [B*F,kmax,7+C] (only local frames' rows are read).
-        `before_cafm(state)` / `after_cafm(state)` let a caller hand the CAFM memory from rank to rank."""
+        `before_cafm(state)` / `after_cafm(state)` let a caller hand the CAFM memory from rank to rank.
+        state_slots: see forward()."""
+        check_state_args(B, kmax, state, resume, state_slots)
+        return self._from_bank(sel, B, F, Lf, kmax, time_embedding, state, resume, trace, status, before_cafm, after_cafm,
+                               state_slots)
+
+    def _from_bank(self, sel, B, F, Lf, kmax, time_embedding, state, resume, trace=None, status=None, before_cafm=None,
+                   after_cafm=None, state_slots=None, cafm_gate=None):
+        """forward_from_bank without the argument checks.  cafm_gate: event the CAFM memory accesses wait for (host path)."""
         cfg, w, dev, dt = self.cfg, self.w, self.device, self.cfg.dtype
         C, D = cfg.num_classes, cfg.dim
         if status is None:
@@ -576,12 +710,17 @@ class AggregationStage:
             if B not in self._zero_resume:
                 self._zero_resume[B] = torch.zeros(B, dtype=torch.int32, device=dev)
             resume = self._zero_resume[B]
+        elif not isinstance(resume, torch.Tensor):
+            resume = torch.tensor([int(x) for x in resume], dtype=torch.int32, device=dev)
+        if state_slots is not None and not (isinstance(state_slots, torch.Tensor) and state_slots.is_cuda):
+            state_slots = torch.tensor([int(x) for x in state_slots], dtype=torch.int32, device=dev)
         if before_cafm is not None:
             before_cafm(state)
         cafm16, cafm32, perm, te32 = self.run_cafm(lay, bank_reg, bank_edge, iou_reg16 if kmax <= 32 else iou_reg32,
                                                    iou_cls16 if kmax <= 32 else iou_cls32, time_embedding, kmax,
                                                    state, resume, status, want_debug=trace is not None, debug=trace,
-                                                   emb16=None if kmax <= 32 else (iou_reg16, iou_cls16))
+                                                   emb16=None if kmax <= 32 else (iou_reg16, iou_cls16),
+                                                   state_slots=state_slots, gate=cafm_gate)
         if after_cafm is not None:
             after_cafm(state)
         f32z = lambda *s: torch.empty(*s, dtype=torch.float32, device=dev)  # noqa: E731  (fully written before read)
@@ -643,8 +782,10 @@ class AggregationStage:
     # ------------------------------------------------------------------------------------------------------
     def run_cafm(self, lay: ops.AttnLayoutT, bank_reg, bank_edge, emb_reg32, emb_cls32, time_embedding, kmax: int,
                  state: CAFMState, resume: torch.Tensor, status: torch.Tensor, want_debug=False, debug: Optional[dict] = None,
-                 emb16=None):
+                 emb16=None, state_slots: Optional[torch.Tensor] = None, gate=None):
         """CAFM (AwarePositionRegMatcher.forward, tscd_matching.py:722-888) for all clips of the batch.
+        state_slots ([B] int32 device tensor, optional): clip b uses slot state_slots[b] of `state` (kernel-side slot map).
+        gate (optional event): the current stream waits for it right before the first kernel that touches `state`.
         emb16 (wide frames): 16-bit copies of the fp32 matching embeddings -> tensor-core cost kernel.
         emb_reg32 / emb_cls32 [loc_cap,1024] are the agg_iou outputs used for matching only: fp32, or -- frames of <= 32
         proposals -- the 16-bit GEMM outputs (fp32 tensors are rounded to the operand type then)."""
@@ -657,7 +798,7 @@ class AggregationStage:
         n_loc_dev = lay.lrow_off[-1:]
         te16 = time_embedding.to(device=dev, dtype=dt).contiguous()
         assert te16.shape == (B * Lf, 256)
-        assert state.slots == B and state.kmax == kmax
+        assert (state.slots == B if state_slots is None else state.slots >= B) and state.kmax == kmax
         _, te32 = ops.linear(te16, w.ape_w, w.ape_b, want16=False, want32=True, tag="time_emb")
         f32z = lambda *s: torch.empty(*s, dtype=torch.float32, device=dev)  # noqa: E731  (fully written before read)
         fast = kmax <= 32            # every frame's working set fits the shared-memory / mma.sync chain (csrc/cafm.cu)
@@ -678,7 +819,9 @@ class AggregationStage:
         perm = torch.empty(loc_cap, dtype=torch.int32, device=dev) if want_debug else None
         cost_full = f32z(B * Lf, kmax, kmax)
         ref_n = torch.empty(B * Lf, dtype=torch.int32, device=dev)
-        ops.call("tscd_cafm_cost", L.CafmCostArgs, B=B, L=Lf, D=D, kmax=kmax, lrow_off=lay.lrow_off, resume=resume,
+        if gate is not None:
+            torch.cuda.current_stream().wait_event(gate)
+        ops.call("tscd_cafm_cost", L.CafmCostArgs, slot=state_slots, B=B, L=Lf, D=D, kmax=kmax, lrow_off=lay.lrow_off, resume=resume,
                  st_n=state.n, emb_reg=emb_reg32, emb_cls=emb_cls32, norm_reg=norm_reg, norm_cls=norm_cls,
                  st_reg=state.reg, st_cls=state.cls, st_nreg=state.nreg, st_ncls=state.ncls, cost=cost_full, ref_n=ref_n,
                  emb_dtype=emb_dtype, emb_reg16=None if emb16 is None else emb16[0], emb_cls16=None if emb16 is None else emb16[1],
@@ -696,7 +839,7 @@ class AggregationStage:
                         dec_w=w.cafm_dec_w, dec_b=w.cafm_dec_b, st_n=state.n, st_out=state.out, st_edge=state.edge,
                         st_reg=state.reg, st_cls=state.cls, st_nreg=state.nreg, st_ncls=state.ncls, st_time=state.time,
                         sc_qin=None, sc_q=None, sc_k=None, ref_n=ref_n, lap_col=lap_col, lap_row=lap_row,
-                        out16=cafm16, out32=cafm32, perm=perm, status=status, emb_dtype=emb_dtype)
+                        out16=cafm16, out32=cafm32, perm=perm, status=status, emb_dtype=emb_dtype, slot=state_slots)
         if fast:
             ops.call("tscd_cafm_chain", L.CafmChainArgs, **chain_kw)
         else:
