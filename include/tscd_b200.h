@@ -30,6 +30,7 @@ extern "C" {
 #define TSCD_ERR_UNSUPPORTED (-2)
 #define TSCD_ERR_CAPACITY (-3)
 #define TSCD_ERR_CUDA (-4)
+#define TSCD_ERR_FRAME_SLOT (-5)   /* device flag of tscd_clip_assemble / tscd_frame_scatter: a frame-store slot out of range or never written */
 
 /* element types of boundary / operand tensors */
 #define TSCD_F32 0
@@ -757,6 +758,57 @@ typedef struct {
     float* v_bank_score;         /* out [rows_cap] */
 } tscd_bank_unpack_args;
 int tscd_bank_unpack(const tscd_bank_unpack_args* args, void* stream);
+
+/* ---- frame store: K1-K3 once per video frame, clips assembled from it on the device ---------------------------------------
+ * Replaces the per-clip repetition of K1-K3 over the frames of tools/tscd_demo.py:223-241 / vid.py:601-683 (each clip = lframe
+ * consecutive local frames + gframe frames drawn from the rest of the video, so a frame appears in many clips).  A caller-owned
+ * store (tscd_b200/frames.py FrameStore) keeps one frame's K1-K3 result per slot at a fixed pitch of kmax rows:
+ *   tscd_frame_scatter   the packed tscd_gather output of N frames (+ tscd_edge_combine's bank_edge) -> slots frame_slots[0..N);
+ *   tscd_clip_assemble   clip_slots [B*F] (clip-major; a slot may repeat, within a clip too) -> exactly the packed clip arrays
+ *                        tscd_gather would have written for those frames: sel_count, row_off (exclusive prefix), bank rows,
+ *                        sel_idx (optional) and the sel_rows of the first L frames of every clip.  Two kernels, no host sync.
+ * A clip slot outside [0, frames) or never written (count -1) sets status to TSCD_ERR_FRAME_SLOT and contributes 0 rows; a slot
+ * written by a call whose status was set passes that code on (K1 / K2 report capacity per call, not per frame).  A frame slot
+ * outside [0, frames) in tscd_frame_scatter sets slot_error to TSCD_ERR_FRAME_SLOT and is skipped (status is only read, so
+ * every written slot carries the same K1-K3 flag whatever the launch order of the blocks).
+ * Banks: 256 16-bit channels per row (TSCD-L); all pointers 16-byte aligned. */
+typedef struct {
+    int32_t frames, kmax, num_classes;
+    int32_t dtype;               /* TSCD_F16 / TSCD_BF16 bank element type */
+    int32_t* count;              /* [frames] kept rows of the frame in the slot, -1 = never written */
+    int32_t* status;             /* [frames] status of the call that wrote the slot (0 = ok) */
+    void* bank_cls; void* bank_reg; void* bank_edge;   /* [frames * kmax, 256] */
+    float* bank_score;           /* [frames * kmax] */
+    int32_t* sel_idx;            /* [frames, kmax] anchor ids */
+    float* sel_rows;             /* [frames, kmax, 7 + num_classes] reference rows */
+} tscd_frame_store;
+
+typedef struct {
+    tscd_frame_store store;
+    int32_t num_frames;          /* N */
+    const int32_t* frame_slots;  /* [N] distinct slots */
+    const int32_t* sel_count; const int32_t* row_off;   /* tscd_gather outputs over the N frames (max_keep == store.kmax) */
+    const int32_t* sel_idx; const float* sel_rows;
+    const void* bank_cls; const void* bank_reg; const void* bank_edge; const float* bank_score;
+    const int32_t* status;       /* [1] the flag K1-K3 of these frames wrote (read only; copied into every slot written) */
+    int32_t* slot_error;         /* [1] optional: set to TSCD_ERR_FRAME_SLOT when a frame slot is outside [0, frames) */
+} tscd_frame_scatter_args;
+int tscd_frame_scatter(const tscd_frame_scatter_args* args, void* stream);
+
+typedef struct {
+    tscd_frame_store store;
+    int32_t B, F, L;
+    int64_t row_cap;             /* rows of the output banks, >= B * F * kmax */
+    const int32_t* clip_slots;   /* [B * F] */
+    int32_t* sel_count;          /* out [B * F] */
+    int32_t* row_off;            /* out [B * F + 1] */
+    void* bank_cls; void* bank_reg; void* bank_edge;   /* out [row_cap, 256] */
+    float* bank_score;           /* out [row_cap] */
+    int32_t* sel_idx;            /* out [B * F, kmax] or NULL */
+    float* sel_rows;             /* out [B * F, kmax, 7 + C]: rows of the local frames written */
+    int32_t* status;             /* [1] */
+} tscd_clip_assemble_args;
+int tscd_clip_assemble(const tscd_clip_assemble_args* args, void* stream);
 
 /* Debug aid: cycles block 0 of the last tscd_cafm_chain launches spent per phase
  * (0 assignment re-index, 1 query input, 2 q projection, 3 normalise, 4 attention, 5 norms/state, 6 state carry). */

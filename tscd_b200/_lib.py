@@ -10,7 +10,9 @@ from .build import LIB_PATH
 
 TSCD_F32, TSCD_F16, TSCD_BF16 = 0, 1, 2
 MAX_LEVELS = 3
-_ERR = {-1: "invalid argument", -2: "unsupported configuration", -3: "capacity exceeded", -4: "CUDA error"}
+_ERR = {-1: "invalid argument", -2: "unsupported configuration", -3: "capacity exceeded", -4: "CUDA error",
+        -5: "frame-store slot out of range or never written"}
+TSCD_ERR_CAPACITY, TSCD_ERR_FRAME_SLOT = -3, -5
 
 
 class View(C.Structure):
@@ -194,6 +196,21 @@ class BankUnpackArgs(C.Structure):
                 ("v_bank_reg", C.c_void_p), ("v_bank_edge", C.c_void_p), ("v_bank_score", C.c_void_p)]
 
 
+class FrameStoreC(C.Structure):
+    _fields_ = _fields("frames:i kmax:i num_classes:i dtype:i count:p status:p bank_cls:p bank_reg:p bank_edge:p bank_score:p "
+                       "sel_idx:p sel_rows:p")
+
+
+class FrameScatterArgs(C.Structure):
+    _fields_ = [("store", FrameStoreC)] + _fields("num_frames:i frame_slots:p sel_count:p row_off:p sel_idx:p sel_rows:p bank_cls:p "
+                                                  "bank_reg:p bank_edge:p bank_score:p status:p slot_error:p")
+
+
+class ClipAssembleArgs(C.Structure):
+    _fields_ = [("store", FrameStoreC), ("B", C.c_int32), ("F", C.c_int32), ("L", C.c_int32), ("row_cap", C.c_int64)] + \
+        _fields("clip_slots:p sel_count:p row_off:p bank_cls:p bank_reg:p bank_edge:p bank_score:p sel_idx:p sel_rows:p status:p")
+
+
 class PackDetectionsArgs(C.Structure):
     _fields_ = _fields("num_frames:i cap:i rows:p count:p scale:p offsets:p packed:p")
 
@@ -250,6 +267,8 @@ SYMBOLS = [
     ("tscd_bank_pack_bytes", C.c_int64, [C.c_int32, C.c_int32]),
     ("tscd_bank_pack", C.c_int, [C.POINTER(BankPackArgs), C.c_void_p]),
     ("tscd_bank_unpack", C.c_int, [C.POINTER(BankUnpackArgs), C.c_void_p]),
+    ("tscd_frame_scatter", C.c_int, [C.POINTER(FrameScatterArgs), C.c_void_p]),
+    ("tscd_clip_assemble", C.c_int, [C.POINTER(ClipAssembleArgs), C.c_void_p]),
 ]
 
 
@@ -272,7 +291,7 @@ def lib():
 
 # kernels launched per C-ABI call (for the bench's `gpu_launches` claim)
 _DEBUG_SYNC = os.environ.get("TSCD_DEBUG_SYNC", "0") == "1"
-KERNELS_PER_CALL = {"tscd_gather": 2, "tscd_nms_large": 3, "tscd_bank_unpack": 2, "tscd_pack_detections": 2, "tscd_pack_rows": 2, "tscd_cafm_wide_p1": 2}
+KERNELS_PER_CALL = {"tscd_gather": 2, "tscd_nms_large": 3, "tscd_bank_unpack": 2, "tscd_clip_assemble": 2, "tscd_pack_detections": 2, "tscd_pack_rows": 2, "tscd_cafm_wide_p1": 2}
 launch_count = 0
 # optional per-entry-point CUDA-event timing: {"names": set or None (= all), "events": {name: [(start, end), ...]}}
 profile = None

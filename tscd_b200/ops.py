@@ -531,3 +531,40 @@ def call(name: str, struct_cls, tag=None, **kw):
     assert not missing, f"{name}: missing {missing}"
     with L.timed(name, tag):
         L.check(getattr(L.lib(), name)(C.byref(a), _stream()), name)
+
+
+# ----------------------------------------------------------------------------------------------- frame store
+def frame_scatter(store, frame_slots: torch.Tensor, sel: dict, status: torch.Tensor, slot_error: Optional[torch.Tensor] = None):
+    """tscd_frame_scatter: the K1-K3 output `sel` of N frames (ops.gather dict, max_keep == store.kmax) -> store slots
+    frame_slots [N] (int32 device tensor).  `status` (the K1-K3 flag) is copied into every slot written; `slot_error` ([1],
+    optional) receives TSCD_ERR_FRAME_SLOT for a slot outside the store.  No host sync."""
+    a = L.FrameScatterArgs()
+    a.store = store.to_c()
+    a.num_frames = frame_slots.numel()
+    a.frame_slots, a.status, a.slot_error = _p(frame_slots), _p(status), _p(slot_error)
+    for k in ("sel_count", "row_off", "sel_idx", "sel_rows", "bank_cls", "bank_reg", "bank_edge", "bank_score"):
+        setattr(a, k, _p(sel[k]))
+    with L.timed("tscd_frame_scatter"):
+        L.check(L.lib().tscd_frame_scatter(C.byref(a), _stream()), "tscd_frame_scatter")
+
+
+def clip_assemble(store, clip_slots: torch.Tensor, B: int, F: int, Lf: int, row_cap: int, status: torch.Tensor,
+                  out: Optional[dict] = None, want_idx: bool = True) -> dict:
+    """tscd_clip_assemble: clip_slots [B, F] (int32 device tensor) -> the packed clip dict forward_from_bank consumes
+    (sel_count, row_off, bank_cls/reg/edge/score with row_cap rows, sel_rows, sel_idx).  `out`: preallocated buffers of that
+    shape to write instead (nothing is allocated then)."""
+    dev = clip_slots.device
+    nf, kmax, W = B * F, store.kmax, 7 + store.num_classes
+    if out is None:
+        out = dict(sel_count=torch.empty(nf, dtype=torch.int32, device=dev),
+                   row_off=torch.empty(nf + 1, dtype=torch.int32, device=dev),
+                   sel_idx=torch.empty(nf, kmax, dtype=torch.int32, device=dev) if want_idx else None,
+                   sel_rows=torch.empty(nf, kmax, W, dtype=torch.float32, device=dev),
+                   bank_score=torch.empty(row_cap, dtype=torch.float32, device=dev), max_keep=kmax)
+        for k in ("bank_cls", "bank_reg", "bank_edge"):
+            out[k] = torch.empty(row_cap, store.dim, dtype=store.dtype, device=dev)
+    call("tscd_clip_assemble", L.ClipAssembleArgs, store=store.to_c(), B=B, F=F, L=Lf, row_cap=out["bank_cls"].shape[0],
+         clip_slots=clip_slots, sel_count=out["sel_count"], row_off=out["row_off"], bank_cls=out["bank_cls"],
+         bank_reg=out["bank_reg"], bank_edge=out["bank_edge"], bank_score=out["bank_score"], sel_idx=out.get("sel_idx"),
+         sel_rows=out["sel_rows"], status=status)
+    return out

@@ -15,12 +15,30 @@ import torch
 
 from . import _lib as L
 from . import aggregate, ops
+from . import frames as _frames
 from . import selection as _selection
 from .selection import SelectionConfig
 
 
 def _r128(x: int) -> int:
     return (x + 127) // 128 * 128
+
+
+class _no_gc_during_capture:
+    """Keeps Python's cyclic garbage collector from running inside a CUDA-graph capture.  torch.cuda.graph collects once on
+    entry, but a collection triggered during the capture can free cyclic garbage of earlier calls (host plans, pinned staging
+    buffers, graphs) whose destructors make CUDA calls that are illegal while a stream is capturing, which aborts the process."""
+
+    def __enter__(self):
+        import gc
+        self.was = gc.isenabled()
+        gc.disable()
+
+    def __exit__(self, *exc):
+        import gc
+        if self.was:
+            gc.enable()
+        return False
 
 
 @dataclass
@@ -59,7 +77,7 @@ def validate_config(cfg: StageConfig):
         raise RuntimeError("more than 255 classes are not supported (8-bit class ids in the selection kernels)")
 
 
-MAX_KEYS_PER_CLIP = 65536     # attention kernels: keys of one clip (csrc/attn.cu, 16-bit key index in row_meta)
+MAX_KEYS_PER_CLIP = _frames.MAX_KEYS_PER_CLIP     # attention kernels: keys of one clip (csrc/attn.cu, 16-bit key index in row_meta)
 
 
 def check_state_args(B: int, kmax: int, state=None, resume=None, state_slots=None, host: bool = False):
@@ -257,9 +275,7 @@ class AggregationStage:
         assert head.num_frames == B * F and 1 <= Lf <= F
         A = head.anchors.num_anchors
         kmax = cfg.selection.max_keep(A)
-        if _r128(F * kmax) > MAX_KEYS_PER_CLIP:
-            raise RuntimeError(f"{F} frames x {kmax} proposals per frame = {F * kmax} keys per clip exceed the attention kernels' "
-                               f"capacity of {MAX_KEYS_PER_CLIP}; lower SelectionConfig.max_proposals")
+        _frames.check_keys_per_clip(F, kmax)
         check_state_args(B, kmax, state, resume, state_slots)
         status = torch.zeros(1, dtype=torch.int32, device=dev)
 
@@ -269,6 +285,87 @@ class AggregationStage:
                                            bank_rows=row_cap)
         return self.forward_from_bank(sel, B, F, Lf, kmax, time_embedding, state=state, resume=resume, trace=trace,
                                       status=status, state_slots=state_slots)
+
+    # ------------------------------------------------------------------------------------------------------
+    def _store_kmax(self, store: _frames.FrameStore, A: Optional[int] = None) -> int:
+        """kmax of this stage for the frames of `store`: A = anchors per frame of the frames at hand (ingest_frames), else those
+        of the frames ingested so far (forward_clips)."""
+        if A is None:
+            if store.num_anchors is None:
+                raise RuntimeError("forward_clips: the FrameStore holds no frames yet; ingest_frames the frames of the clips first")
+            A = store.num_anchors
+        elif store.num_anchors not in (None, A):
+            raise RuntimeError(f"ingest_frames: the FrameStore holds frames of {store.num_anchors} anchors, these frames have {A}; "
+                               "one store holds frames of one input size")
+        return self.cfg.selection.max_keep(A)
+
+    def ingest_frames(self, store: _frames.FrameStore, head: ops.HeadViews, feats, feat_dtype, frame_slots):
+        """K1-K3 (selection, pre-NMS, bank gather, edge rows) ONCE for N video frames, written into the slots `frame_slots` of
+        `store` (tscd_frame_scatter).  head / feats: the N frames in any layout forward() accepts (fused rows, per level,
+        row-major, or an EdgeBlock as feats[2]).  frame_slots: [N] distinct slots (a list, or an int32 device tensor -- then
+        nothing is read back and the call can be captured into a CUDA graph).  Returns the K1-K3 output of the N frames: its
+        'status' is the flag every written slot carries (a capacity error shows up in the clips that use these frames), and
+        'slot_error' ([1] int32, device) is TSCD_ERR_FRAME_SLOT when a device-tensor slot lay outside the store -- such a frame is
+        not written, and nothing else reports it (host-side slots are checked before any launch).
+        Capacity flags are per call, not per frame: ingesting a video in several calls narrows which clips an overflow stops."""
+        cfg, dev, dt = self.cfg, self.device, self.cfg.dtype
+        A, N = head.anchors.num_anchors, head.num_frames
+        kmax = self._store_kmax(store, A)
+        _frames.check_clip_args(store, frame_slots, kmax, cfg.num_classes, cfg.dim, dt, num_frames=N)
+        store.num_anchors = A
+        slots = self._slot_tensor(frame_slots)
+        status = torch.zeros(1, dtype=torch.int32, device=dev)
+        sel = _selection.select_and_gather(head, feats, feat_dtype, cfg.dim, cfg.selection, bank_dtype=dt, status=status,
+                                           bank_rows=_r128(N * kmax) + 128)
+        sel["slot_error"] = torch.zeros(1, dtype=torch.int32, device=dev)
+        ops.frame_scatter(store, slots, sel, status, sel["slot_error"])
+        return sel
+
+    def ingest_host_frames(self, store: _frames.FrameStore, host: dict, hw, frame_slots, strides=(8, 16, 32)):
+        """ingest_frames for N frames in PINNED HOST memory, in the fused-row layout forward_host reads: host['rows'] = [rows
+        [N, A, 32|64] fp16], host['objp'] = [objectness plane [N, >=A]], host['f_cls' / 'f_reg' / 'f_edge'] = per-level
+        [N, 256, H, W] channels_last planes.  As in forward_host, the objectness plane is copied; in mode A, K1 / K3 read the
+        survivors' rows in place, mode B copies the rows; K3 reads the kept proposals' feature rows in place (UVA).  So each
+        frame crosses PCIe once however many clips use it.  Eager launches, no host sync.  Returns (K1-K3 output, bytes
+        copied host->device); the bytes read in place follow from the counts (tools/bench_frame_store.py)."""
+        an = ops.AnchorSpec(hw, strides)
+        if "rows" not in host:
+            raise RuntimeError("ingest_host_frames: host frames must be in the fused-row layout (host['rows'], host['objp'])")
+        for k in ("rows", "objp", "f_cls", "f_reg", "f_edge"):
+            for t in host[k]:
+                if t.device.type != "cpu" or not t.is_pinned():
+                    raise RuntimeError(f"ingest_host_frames: host['{k}'] must be pinned CPU tensors (cudaHostAlloc) so the GPU can "
+                                       "read them in place; there is no pageable-memory / CPU path")
+        rows_in_place = self.cfg.selection.mode == "A"
+        copied = ("objp",) if rows_in_place else ("objp", "rows")
+        dbuf = {k: host[k][0].to(self.device, non_blocking=True) for k in copied}
+        h2d = sum(host[k][0].numel() * host[k][0].element_size() for k in copied)
+        head = ops.HeadViews.from_rows(host["rows"][0] if rows_in_place else dbuf["rows"], dbuf["objp"], an, self.cfg.num_classes)
+        feats = tuple(ops.view_levels(host[k]) for k in ("f_cls", "f_reg", "f_edge"))
+        return self.ingest_frames(store, head, feats, host["f_cls"][0].dtype, frame_slots), h2d
+
+    def forward_clips(self, store: _frames.FrameStore, clip_slots, Lf: int, time_embedding: torch.Tensor,
+                      state: Optional[CAFMState] = None, resume=None, state_slots=None):
+        """The stage for B clips whose frames are in `store` (ingest_frames): clip_slots [B, F] holds the slot of every frame of
+        every clip, local frames first (a slot may repeat, within a clip too).  tscd_clip_assemble rebuilds the packed clip bank
+        K1-K3 would have produced for those frames, then forward_from_bank runs the rest; the result is the dict forward()
+        returns (to_lists works unchanged), bit for bit.  clip_slots as an int32 device tensor: nothing is read back, and the
+        call can be captured (capture_fn) and replayed with refilled slots.  state / resume / state_slots: as in forward()."""
+        cfg, dt = self.cfg, self.cfg.dtype
+        kmax = self._store_kmax(store)
+        _frames.check_clip_args(store, clip_slots, kmax, cfg.num_classes, cfg.dim, dt, L=Lf)
+        slots = self._slot_tensor(clip_slots)
+        B, F = slots.shape
+        check_state_args(B, kmax, state, resume, state_slots)
+        status = torch.zeros(1, dtype=torch.int32, device=self.device)
+        sel = ops.clip_assemble(store, slots, B, F, Lf, _r128(B * F * kmax) + 128, status)
+        return self._from_bank(sel, B, F, Lf, kmax, time_embedding, state, resume, status=status, state_slots=state_slots)
+
+    def _slot_tensor(self, slots) -> torch.Tensor:
+        if isinstance(slots, torch.Tensor) and slots.is_cuda:
+            return slots
+        return torch.tensor(np.asarray(slots.cpu() if isinstance(slots, torch.Tensor) else slots, dtype=np.int32),
+                            dtype=torch.int32, device=self.device)
 
     # ------------------------------------------------------------------------------------------------------
     def forward_host(self, host: dict, hw, time_embedding: torch.Tensor, B: int, F: int, Lf: int, chunk_clips: int = 8,
@@ -536,7 +633,7 @@ class AggregationStage:
             torch.cuda.current_stream().wait_stream(hp)
             torch.cuda.synchronize()
             g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g, stream=hp):
+            with _no_gc_during_capture(), torch.cuda.graph(g, stream=hp):
                 issue(pool)
             plan["graph"] = g
         return plan
@@ -619,7 +716,7 @@ class AggregationStage:
         torch.cuda.current_stream().wait_stream(s)
         torch.cuda.synchronize()
         graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(graph):
+        with _no_gc_during_capture(), torch.cuda.graph(graph):
             out = self.forward(head, feats, feat_dtype, te, B, F, Lf, state=state, resume=resume, state_slots=state_slots)
         if state_slots is not None:
             out["state_slots"] = state_slots
@@ -641,7 +738,7 @@ class AggregationStage:
         torch.cuda.current_stream().wait_stream(hp)
         torch.cuda.synchronize()
         graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(graph, stream=hp):
+        with _no_gc_during_capture(), torch.cuda.graph(graph, stream=hp):
             out = fn()
         return graph, out
 
@@ -895,6 +992,9 @@ class AggregationStage:
         """One device->host read; returns (result, result_ori) with the reference's container types
         (post_process.py:12-13,85): per local frame a fresh Tensor[n,7] or None."""
         st = int(out["status"].item())
+        if st == L.TSCD_ERR_FRAME_SLOT:
+            raise RuntimeError(f"tscd_b200 stage reported error {st} (a clip references a frame-store slot that was never written "
+                               "or lies outside the FrameStore: ingest_frames every frame of the clips before forward_clips)")
         if st != 0:
             raise RuntimeError(f"tscd_b200 stage reported error {st} (capacity exceeded: a frame holds more proposals than "
                                f"the per-frame capacity of {out['sel']['sel_rows'].shape[1]} -- raise SelectionConfig.max_proposals "
