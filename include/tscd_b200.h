@@ -304,7 +304,7 @@ typedef struct {
     const float* key_score;   /* [rows] or NULL (reg branch) */
     float scale;              /* 25 */
     void *qn, *kn, *vn;       /* [rows,256] */
-    void* vt;                 /* [B*256, nk_pitch] */
+    void* vt;                 /* [B*256, nk_pitch], or NULL: not computed (the reg branch of a module run with need_reg = 0) */
     void* xori;               /* [loc_cap, ld_xori] or NULL */
     int32_t ld_xori;
 } tscd_qkv_project_args;
@@ -322,7 +322,7 @@ int tscd_attn_rowmeta(const tscd_attn_rowmeta_args* args, void* stream);
 typedef struct {
     tscd_attn_layout lay;
     const void *qn_cls, *kn_cls, *qn_reg, *kn_reg;
-    const void *vt_cls, *vt_reg;
+    const void *vt_cls, *vt_reg;   /* vt_reg may be NULL when need_reg = 0 */
     const int32_t* row_frame;
     int32_t need_reg;         /* 0: skip attn @ v_reg (TSCD `agg` discards it, tscd_head.py:480) */
     void* x_cls;              /* [loc_cap, ld_x] attn @ v_cls, heads concatenated */

@@ -67,8 +67,10 @@ def mca_forward(lay: ops.AttnLayoutT, w: MCAWeights, bank_cls, bank_reg, bank_sc
     tmp_r = torch.empty(lay.loc_cap, 512, dtype=dt, device=dev)
     qkv_c = qkv_r = None
     if FUSED_QKV:
+        # without need_reg nothing reads the reg branch's V^T or x_ori (only attn_pv's reg-value product and linear_reg do)
         bufs = ops.qkv_project_fused(lay, bank_cls, bank_reg, w.qkv_cls, w.qkv_reg, bank_score, n_rows_dev,
-                                     xori_cls=tmp_c[:, 256:], xori_reg=tmp_r[:, 256:], tag=tag)
+                                     xori_cls=tmp_c[:, 256:], xori_reg=tmp_r[:, 256:] if need_reg else None, tag=tag,
+                                     need_reg=need_reg)
     else:
         qkv_c, _ = ops.linear(bank_cls, w.qkv_cls, m_dev=n_rows_dev)
         qkv_r, _ = ops.linear(bank_reg, w.qkv_reg, m_dev=n_rows_dev)

@@ -1151,7 +1151,9 @@ extern "C" int tscd_attn_pv(const tscd_attn_pv_args* a, void* stream) {
     rc |= make_tmap_kmajor(&tm.k64c, a->kn_cls, bf, l.row_cap, 256, 256, 64);
     rc |= make_tmap_kmajor(&tm.k64r, a->kn_reg, bf, l.row_cap, 256, 256, 64);
     rc |= make_tmap_kmajor(&tm.vtc, a->vt_cls, bf, (int64_t)l.B * 256, l.nk_pitch, l.nk_pitch, 64);
-    rc |= make_tmap_kmajor(&tm.vtr, a->vt_reg, bf, (int64_t)l.B * 256, l.nk_pitch, l.nk_pitch, 64);
+    if (a->need_reg && !a->vt_reg) return TSCD_ERR_INVALID_ARG;
+    // without need_reg the reg V^T is never loaded (and may be NULL): its map points at vt_cls
+    rc |= make_tmap_kmajor(&tm.vtr, a->need_reg ? a->vt_reg : a->vt_cls, bf, (int64_t)l.B * 256, l.nk_pitch, l.nk_pitch, 64);
     if (rc) return TSCD_ERR_CUDA;
     const size_t smem = 65536 + kPvStages * 32768 + 65536 + sizeof(PvBars);
     dim3 grid((l.nk_pitch + 127) / 128, l.B);      // query tiles are bounded by the clip size; empty tiles exit at once

@@ -39,7 +39,7 @@ struct GemmParams {
     const int32_t* row_meta;   // [rows] (clip << 16) | key index within the clip
     const int32_t* row_off;    // [B*F+1]
     const int32_t* lrow_off;   // [B*L+1]
-    int F, L, self_attn, nk_pitch;
+    int B, F, L, self_attn, nk_pitch;
     const float* key_score;    // [rows] or NULL
     float scale;
     void *qn, *kn, *vn, *vt, *xori;
@@ -70,6 +70,18 @@ __device__ __forceinline__ void gemm_wait_prof(uint64_t* bar, uint32_t parity, i
 // weight load (192 KB -> 64 KB of L2 -> shared-memory traffic per tile).
 constexpr int kAccStages = 2;
 
+// Fused q|k|v projection (EPI = 1) schedule: the grid is G groups of 3 CTAs.  Group g walks m-tiles g, g + G, g + 2G, ...
+// in rounds; in every round its three CTAs compute the q, k and v tiles of the same 128 bank rows at the same time, so
+// those rows come from DRAM once and the other two CTAs read them from L2 (the m-fastest order of the plain kernel reads
+// every row three times: all q tiles, then all k tiles, then all v tiles).  CTA j of a group computes column block
+// (j + phase) % 3, where the phase (0, 1, 2) is the third of the rounds the round falls in: every CTA keeps one weight
+// tile resident for a third of its tiles and gets an equal share of the three epilogues (v writes V^T and x_ori too).
+// q is only stored for query rows (the first L frames of a clip), so a q tile without one is skipped altogether: no
+// loads, MMA or epilogue.  The CTA then moves on to its next round.  Which of its q rounds hold a query row is worked out
+// once at kernel start into a byte per round (rounds beyond kQFlagCap, i.e. more than 2048 x 49 m-tiles, are not skipped).
+constexpr int kQkvGroup = 3;
+constexpr int kQFlagCap = 2048;
+
 template <int BN, bool BF16, int EPI = 0>
 __global__ void __launch_bounds__(EPI ? kGemmThreadsFused : kGemmThreads) gemm_tn_kernel(const __grid_constant__ CUtensorMap tmap_a,
                                                                 const __grid_constant__ CUtensorMap tmap_w,
@@ -81,7 +93,12 @@ __global__ void __launch_bounds__(EPI ? kGemmThreadsFused : kGemmThreads) gemm_t
     const int tiles_n = (p.N + BN - 1) / BN;
     const int tiles_m = (M + kGemmBM - 1) / kGemmBM;      // only tiles with valid rows exist
     const int num_tiles = tiles_m * tiles_n;
-    if ((int)blockIdx.x >= num_tiles) return;             // uniform over the CTA, before any barrier / TMEM state exists
+    // EPI = 1: group, member and round count of the grouped schedule (the host launches a multiple of 3 CTAs)
+    const int groups = EPI ? (int)gridDim.x / kQkvGroup : 0;
+    const int grp = EPI ? (int)blockIdx.x / kQkvGroup : 0, member = EPI ? (int)blockIdx.x % kQkvGroup : 0;
+    const int rounds = EPI ? (tiles_m + groups - 1) / groups : 0;
+    // uniform over the CTA, before any barrier / TMEM state exists
+    if (EPI ? grp >= tiles_m : (int)blockIdx.x >= num_tiles) return;
 #ifdef TSCD_R2_PROF
     const long long tk0 = clock64();
 #endif
@@ -106,10 +123,30 @@ __global__ void __launch_bounds__(EPI ? kGemmThreadsFused : kGemmThreads) gemm_t
     const int lane = threadIdx.x & 31;
     const int num_kb = (p.K + kGemmBK - 1) / kGemmBK;
     const bool w_resident = num_kb == STAGES;
-    auto tile_origin = [&](int t, int& m0, int& n0) {
-        if (w_resident) { m0 = (t % tiles_m) * kGemmBM; n0 = (t / tiles_m) * BN; }
-        else { m0 = (t / tiles_n) * kGemmBM; n0 = (t % tiles_n) * BN; }
+    unsigned char* qflag = reinterpret_cast<unsigned char*>(full_bar) + 128;   // EPI = 1: [kQFlagCap] per round
+    // The CTA's next tile: `cur` is the tile index (plain kernel) or the round (EPI = 1); false when the CTA is done.
+    // Every role of the CTA walks the same sequence with its own cursor.
+    auto next_tile = [&](int& cur, int& m0, int& n0) -> bool {
+        if constexpr (EPI == 1) {
+            for (;; ++cur) {
+                const int mt = grp + groups * cur;
+                if (mt >= tiles_m) return false;
+                const int kind = (member + kQkvGroup * cur / rounds) % kQkvGroup;
+                if (kind == 0 && cur < kQFlagCap && !qflag[cur]) continue;
+                m0 = mt * kGemmBM;
+                n0 = kind * BN;
+                ++cur;
+                return true;
+            }
+        } else {
+            if (cur >= num_tiles) return false;
+            if (w_resident) { m0 = (cur % tiles_m) * kGemmBM; n0 = (cur / tiles_m) * BN; }
+            else { m0 = (cur / tiles_n) * kGemmBM; n0 = (cur % tiles_n) * BN; }
+            cur += gridDim.x;
+            return true;
+        }
     };
+    const int cur0 = EPI ? 0 : (int)blockIdx.x;
 
     if (warp == 0 && lane == 0) {
         tma_prefetch_desc(&tmap_a);
@@ -119,6 +156,30 @@ __global__ void __launch_bounds__(EPI ? kGemmThreadsFused : kGemmThreads) gemm_t
         fence_barrier_init();
     }
     if (warp == 1) tmem_alloc<kAccStages * BN>(&tmem_base_smem);
+    if constexpr (EPI == 1) {
+        // epilogue threads: does the q tile of round r hold a query row?  Rows [row_off[c*F], row_off[c*F+L]) of clip c
+        // are its queries (the whole clip for self-attention); walk the clips that start inside the tile.
+        if (warp >= 2) {
+            for (int r = threadIdx.x - 64; r < min(rounds, kQFlagCap); r += blockDim.x - 64) {
+                const int mt = grp + groups * r;
+                bool hq = true;
+                if (mt < tiles_m && (member + kQkvGroup * r / rounds) % kQkvGroup == 0) {
+                    const int m_end = min(M, (mt + 1) * kGemmBM);
+                    int row = mt * kGemmBM;
+                    const int meta = __ldg(p.row_meta + row);
+                    if (meta >= 0) {
+                        hq = false;
+                        for (int cb = meta >> 16; row < m_end && cb < p.B; ++cb) {
+                            const int qend = __ldg(p.row_off + (p.self_attn ? (cb + 1) * p.F : cb * p.F + p.L));
+                            if (row < qend) { hq = true; break; }
+                            row = __ldg(p.row_off + (cb + 1) * p.F);
+                        }
+                    }
+                }
+                qflag[r] = hq;
+            }
+        }
+    }
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -128,9 +189,8 @@ __global__ void __launch_bounds__(EPI ? kGemmThreadsFused : kGemmThreads) gemm_t
         if (lane == 0) {
             uint32_t it = 0;   // running k-block counter across tiles -> ring stage / phase
             int n_prev = -1;   // column block whose weights the stages hold (w_resident)
-            for (int t = blockIdx.x; t < num_tiles; t += gridDim.x) {
-                int m0, n0;
-                tile_origin(t, m0, n0);
+            int cur = cur0, m0, n0;
+            while (next_tile(cur, m0, n0)) {
                 const bool load_w = !(w_resident && n0 == n_prev);
                 for (int kb = 0; kb < num_kb; ++kb, ++it) {
                     const int s = it % STAGES;
@@ -148,7 +208,8 @@ __global__ void __launch_bounds__(EPI ? kGemmThreadsFused : kGemmThreads) gemm_t
             // loop in front of every tcgen05.mma), one elected lane issues
             const uint32_t idesc = make_idesc_f16(BF16, kGemmBM, BN);
             uint32_t it = 0, ti = 0;
-            for (int t = blockIdx.x; t < num_tiles; t += gridDim.x, ++ti) {
+            int cur = cur0, m0, n0;
+            for (; next_tile(cur, m0, n0); ++ti) {
                 const int acc = ti % kAccStages;
                 const uint32_t aph = (ti / kAccStages) & 1;
                 GEMM_WAIT(&tmem_empty_bar[acc], aph ^ 1, 130 + acc, 1);     // epilogue has drained this accumulator
@@ -185,9 +246,8 @@ __global__ void __launch_bounds__(EPI ? kGemmThreadsFused : kGemmThreads) gemm_t
         const bool al16 = p.out16 && (p.ld16 % 8) == 0 && (reinterpret_cast<uintptr_t>(p.out16) & 15) == 0;
         const bool al32 = p.out32 && (p.ld32 % 4) == 0 && (reinterpret_cast<uintptr_t>(p.out32) & 15) == 0;
         uint32_t ti = 0;
-        for (int t = blockIdx.x; t < num_tiles; t += gridDim.x, ++ti) {
-            int m0, n0;
-            tile_origin(t, m0, n0);
+        int cur = cur0, m0, n0;
+        for (; next_tile(cur, m0, n0); ++ti) {
             const int acc = ti % kAccStages;
             const uint32_t aph = (ti / kAccStages) & 1;
             const int row_base = m0 + q * 32;
@@ -274,7 +334,7 @@ __global__ void __launch_bounds__(EPI ? kGemmThreadsFused : kGemmThreads) gemm_t
                             for (int j = 0; j < 16; ++j) w16[j] = pk2h(__uint_as_float(r1[2 * j]), __uint_as_float(r1[2 * j + 1]));
                             staged_store(w16, reinterpret_cast<uint16_t*>(p.xori), xdest, p.ld_xori, head * 64 + 32);
                         }
-                        if (valid) {
+                        if (valid && p.vt) {
                             uint16_t* vt = reinterpret_cast<uint16_t*>(p.vt) + ((int64_t)cb * 256 + head * 64) * p.nk_pitch + kr;
 #pragma unroll
                             for (int j = 0; j < 32; ++j) {
@@ -426,7 +486,8 @@ int make_tmap_kmajor(CUtensorMap* m, const void* ptr, int is_bf16, int64_t rows,
 template <int BN, bool BF16, int EPI = 0>
 static int launch_gemm(const CUtensorMap& ta, const CUtensorMap& tw, const GemmParams& p, cudaStream_t st) {
     constexpr int STAGES = BN == 256 ? 4 : 3;
-    constexpr size_t smem = (size_t)STAGES * (kGemmBM * kGemmBK * 2 + BN * kGemmBK * 2) + gemm_epi_warps(EPI) * 2048 + 128;
+    constexpr size_t smem = (size_t)STAGES * (kGemmBM * kGemmBK * 2 + BN * kGemmBK * 2) + gemm_epi_warps(EPI) * 2048 + 128 +
+                            (EPI ? kQFlagCap : 0);   // 229504 + 2048 bytes for the fused projection, under the 227 KB limit
     // per-DEVICE caches (the attribute is per device; a process may drive several GPUs)
     static bool attr_set[64] = {};
     static int num_sms_dev[64] = {};
@@ -441,7 +502,11 @@ static int launch_gemm(const CUtensorMap& ta, const CUtensorMap& tw, const GemmP
     const int num_sms = num_sms_dev[dev];
     const int tiles = ((p.N + BN - 1) / BN) * ((p.M + kGemmBM - 1) / kGemmBM);
     const int ctas_per_sm = BN == 256 ? 1 : 2;                       // 113 KB smem and 2*BN TMEM columns per CTA (BN <= 128)
-    const int grid = tiles < ctas_per_sm * num_sms ? tiles : ctas_per_sm * num_sms;
+    int grid = tiles < ctas_per_sm * num_sms ? tiles : ctas_per_sm * num_sms;
+    if (EPI) {   // whole groups of kQkvGroup CTAs, at most one group per m-tile
+        const int tiles_m = (p.M + kGemmBM - 1) / kGemmBM;
+        grid = kQkvGroup * min(tiles_m, num_sms / kQkvGroup);
+    }
     gemm_tn_kernel<BN, BF16, EPI><<<grid, EPI ? kGemmThreadsFused : kGemmThreads, smem, st>>>(ta, tw, p);
     return cudaGetLastError() == cudaSuccess ? TSCD_OK : TSCD_ERR_CUDA;
 }
@@ -476,7 +541,7 @@ extern "C" int tscd_linear(const tscd_linear_args* a, void* stream) {
 
 extern "C" int tscd_qkv_project(const tscd_qkv_project_args* a, void* stream) {
     using namespace tscd;
-    if (!a || a->rows <= 0 || !a->x || !a->w || !a->row_meta || !a->qn || !a->kn || !a->vn || !a->vt) return TSCD_ERR_INVALID_ARG;
+    if (!a || a->rows <= 0 || !a->x || !a->w || !a->row_meta || !a->qn || !a->kn || !a->vn) return TSCD_ERR_INVALID_ARG;
     const tscd_attn_layout& l = a->lay;
     if (l.dtype != TSCD_F16 && l.dtype != TSCD_BF16) return TSCD_ERR_UNSUPPORTED;
     if (l.B <= 0 || l.F <= 0 || l.L <= 0 || l.L > l.F || !l.row_off || !l.lrow_off || (l.nk_pitch % 128) != 0 || l.nk_pitch > 65536) return TSCD_ERR_INVALID_ARG;
@@ -491,7 +556,7 @@ extern "C" int tscd_qkv_project(const tscd_qkv_project_args* a, void* stream) {
     p.m_dev = a->m_dev;
     p.is_bf16 = is_bf16;
     p.row_meta = a->row_meta; p.row_off = l.row_off; p.lrow_off = l.lrow_off;
-    p.F = l.F; p.L = l.L; p.self_attn = l.self_attn; p.nk_pitch = l.nk_pitch;
+    p.B = l.B; p.F = l.F; p.L = l.L; p.self_attn = l.self_attn; p.nk_pitch = l.nk_pitch;
     p.key_score = a->key_score; p.scale = a->scale;
     p.qn = a->qn; p.kn = a->kn; p.vn = a->vn; p.vt = a->vt; p.xori = a->xori; p.ld_xori = a->ld_xori;
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);

@@ -465,24 +465,27 @@ def attn_prep(lay: AttnLayoutT, qkv_cls, qkv_reg, key_score, xori_cls=None, xori
 
 
 def qkv_project_fused(lay: AttnLayoutT, bank_cls, bank_reg, w_cls, w_reg, key_score, n_rows_dev, xori_cls=None, xori_reg=None,
-                      scale=25.0, tag=None):
+                      scale=25.0, tag=None, bufs=None, need_reg=True):
     """tscd_attn_rowmeta + 2 x tscd_qkv_project: the q|k|v projections of both branches with the normalise / scale /
-    transpose step of tscd_attn_prep fused into the GEMM epilogue.  Returns the same operand dict as attn_prep."""
+    transpose step of tscd_attn_prep fused into the GEMM epilogue.  Returns the same operand dict as attn_prep (plus
+    row_meta); `bufs` may supply that dict's buffers.  need_reg=False: a module whose attention never reads the reg
+    branch's V^T (attn_pv / mca_forward with need_reg=False): no vt_reg is allocated or computed; pass xori_reg=None too."""
     dev, dt = bank_cls.device, lay.dtype
-    bufs = {}
-    for n in ("qn_cls", "kn_cls", "vn_cls", "qn_reg", "kn_reg", "vn_reg"):
-        bufs[n] = torch.empty(lay.row_cap, 256, dtype=dt, device=dev)
-    for n in ("vt_cls", "vt_reg"):
-        bufs[n] = torch.empty(lay.B * 256, lay.nk_pitch, dtype=dt, device=dev)
-    bufs["row_frame"] = torch.empty(lay.row_cap, dtype=torch.int32, device=dev)
-    bufs["row_meta"] = torch.empty(lay.row_cap, dtype=torch.int32, device=dev)
+    if bufs is None:
+        bufs = {}
+        for n in ("qn_cls", "kn_cls", "vn_cls", "qn_reg", "kn_reg", "vn_reg"):
+            bufs[n] = torch.empty(lay.row_cap, 256, dtype=dt, device=dev)
+        for n in ("vt_cls", "vt_reg")[:2 if need_reg else 1]:
+            bufs[n] = torch.empty(lay.B * 256, lay.nk_pitch, dtype=dt, device=dev)
+        bufs["row_frame"] = torch.empty(lay.row_cap, dtype=torch.int32, device=dev)
+        bufs["row_meta"] = torch.empty(lay.row_cap, dtype=torch.int32, device=dev)
     call("tscd_attn_rowmeta", L.AttnRowmetaArgs, lay=lay.to_c(), row_frame=bufs["row_frame"], row_meta=bufs["row_meta"],
-         vt_cls=bufs["vt_cls"], vt_reg=bufs["vt_reg"])
+         vt_cls=bufs["vt_cls"], vt_reg=bufs.get("vt_reg"))
     for br, bank, w, ks, xo in (("cls", bank_cls, w_cls, key_score, xori_cls), ("reg", bank_reg, w_reg, None, xori_reg)):
         assert bank.shape[0] >= lay.row_cap and bank.stride(1) == 1 and w.shape == (768, 256) and w.is_contiguous()
         call("tscd_qkv_project", L.QkvProjectArgs, tag=None if tag is None else f"{tag}.{br}", lay=lay.to_c(), rows=lay.row_cap, m_dev=n_rows_dev, x=bank, ldx=bank.stride(0),
              w=w, row_meta=bufs["row_meta"], key_score=ks, scale=scale, qn=bufs["qn_" + br], kn=bufs["kn_" + br],
-             vn=bufs["vn_" + br], vt=bufs["vt_" + br], xori=xo, ld_xori=0 if xo is None else xo.stride(0))
+             vn=bufs["vn_" + br], vt=bufs.get("vt_" + br), xori=xo, ld_xori=0 if xo is None else xo.stride(0))
     return bufs
 
 
@@ -492,7 +495,7 @@ def attn_pv(lay: AttnLayoutT, bufs, x_cls, x_reg, stats, need_reg=True, tag=None
     a.max_logit = max_logit
     a.lay = lay.to_c()
     for n in ("qn_cls", "kn_cls", "qn_reg", "kn_reg", "vt_cls", "vt_reg", "row_frame"):
-        setattr(a, n, _p(bufs[n]))
+        setattr(a, n, _p(bufs.get(n)))
     a.need_reg = int(need_reg)
     a.x_cls, a.x_reg, a.ld_x, a.stats = _p(x_cls), _p(x_reg), x_cls.stride(0), _p(stats)
     with L.timed("tscd_attn_pv", tag):
