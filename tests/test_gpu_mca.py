@@ -1,7 +1,9 @@
 """GPU parity: K4 cross-frame attention aggregation (tcgen05) vs the oracle's restatement of
-MCA_tscd_g2l_reg / Attention_mca_g2l.  Tolerance: max error relative to the tensor's max <= 1e-2
-(north_star; fp16 operands, fp32 accumulation), with rows whose thresholded cosine similarity is within
-2e-3 of 0.75 / 0.99 in the oracle excluded from the round-2 comparison (discrete flips are expected there)."""
+MCA_tscd_g2l_reg / Attention_mca_g2l and MSA_yolov, at module level (after the output Linears).  Tolerance: max error
+relative to the tensor's max <= 1e-2 (north_star; 16-bit operands, fp32 accumulation), no rows excluded.  For clustered
+features the ragged-clip test does not compare with the oracle at all -- their similarities sit at the 0.75 / 0.99
+thresholds, where the masks may flip -- and checks only that two runs are bit-identical and finite.  The kernels
+themselves are checked element by element, masks included, in test_gpu_attn_kernels.py."""
 import pytest
 import torch
 

@@ -1,8 +1,16 @@
-"""GPU: the fused q|k|v projection (tscd_qkv_project) at the stage's batch shapes.  Every element that the attention
-kernels and the MCA linear read must be written: qn of query rows, kn / vn of every row, V^T with its zeroed pad
-columns up to the next multiple of 128, x_ori of query rows.  The outputs are checked against the unfused pair
-(tscd_linear + tscd_attn_prep) within fp16 tolerance, starting from buffers filled with NaN, and repeated launches must
-give identical bytes, also with need_reg=False (the `agg` module), which leaves out the reg branch's V^T and x_ori."""
+"""GPU: the fused q|k|v projection (tscd_qkv_project) at the stage's batch shapes, fp16 and BF16.  Every element that the
+attention kernels and the MCA linear read must be written: qn of query rows, kn / vn of every row, V^T with its zeroed pad
+columns up to the next multiple of 128, x_ori of query rows.  Both the fused projection and the unfused pair (tscd_linear +
+tscd_attn_prep) are checked element by element against a float64 reference of the same 16-bit bank and weights --
+per-head L2 normalisation without epsilon, 25 * score folded into kn_cls and 25 into kn_reg, raw v in V^T and x_ori --
+starting from buffers filled with NaN, and repeated launches must give identical bytes, also with need_reg=False (the `agg`
+module), which leaves out the reg branch's V^T and x_ori.
+
+Bound (u = 2^-11 fp16, 2^-8 BF16): the GEMM sums 256 products in fp32, so an output y_k of x @ w^T is within
+e_k = 256 * 2^-23 * (|x| @ |w|^T)_k of exact (one ulp per addition).  Raw v: |v - ref| <= e + u|ref| (16-bit store).  A
+per-head normalised output s * y / |y| moves by at most 2 s |e_h| / |y_h| (|e_h| the norm of e over the head) plus the
+16-bit store u s |ref|; the unfused pair first stores y in 16 bits, which adds 2 u s, and a few fp32 ulp of s cover the
+norm itself."""
 import numpy as np
 import pytest
 import torch
@@ -26,10 +34,32 @@ def _counts(case, rng):
     return 7, 5, 2, c.tolist()
 
 
+U = {torch.float16: 2.0 ** -11, torch.bfloat16: 2.0 ** -8}
+
+
+def _reference(x, w, key_score, scale):
+    """float64 (qn, kn, v) of one branch plus their error bounds' ingredients, rows of x."""
+    x, w = x.double(), w.double()
+    y = x @ w.T
+    e = 256 * 2.0 ** -23 * (x.abs() @ w.abs().T)
+    out = {}
+    for name, c0, s in (("qn", 0, torch.ones(x.shape[0], 1, dtype=torch.float64, device=x.device)),
+                        ("kn", 256, scale * (key_score.double()[:, None] if key_score is not None else 1.0) * torch.ones(x.shape[0], 1, dtype=torch.float64, device=x.device)),
+                        ("vn", 512, torch.ones(x.shape[0], 1, dtype=torch.float64, device=x.device))):
+        yh, eh = y[:, c0:c0 + 256].view(-1, 4, 64), e[:, c0:c0 + 256].view(-1, 4, 64)
+        nrm = yh.norm(dim=-1, keepdim=True)
+        out[name] = ((yh / nrm) * s[:, :, None]).reshape(-1, 256)
+        out[name + "_err"] = (2 * eh.norm(dim=-1, keepdim=True) / nrm * s[:, :, None]).expand(-1, 4, 64).reshape(-1, 256)
+        out[name + "_scale"] = s
+    out["v"], out["v_err"] = y[:, 512:], e[:, 512:]
+    return out
+
+
+@pytest.mark.parametrize("dtype", [torch.float16, torch.bfloat16], ids=["fp16", "bf16"])
 @pytest.mark.parametrize("case", ["headline", "ovis_l_ragged", "vid_l", "straddle"])
-def test_qkv_project_matches_unfused(case):
+def test_qkv_project_matches_unfused(case, dtype):
     from tscd_b200 import aggregate, ops
-    dt = torch.float16
+    dt = dtype
     rng = np.random.default_rng(7)
     B, F, L, counts = _counts(case, rng)
     N = sum(counts)
@@ -75,24 +105,39 @@ def test_qkv_project_matches_unfused(case):
     starts = np.concatenate([[0], np.cumsum(clip_rows)])
     qrows = torch.from_numpy(np.concatenate([np.arange(starts[b], starts[b] + loc_rows[b]) for b in range(B)])).cuda()
 
-    def check(name, got, want):
-        got, want = got.float(), want.float()
-        assert not torch.isnan(got).any(), f"{case}: {name} has elements the projection never wrote"
-        err = float((got - want).abs().max() / want.abs().max().clamp_min(1e-6))
-        assert err < 5e-3, f"{case}: {name} max relative error {err:.2e}"
+    u = U[dt]
+    worst = {}
 
-    for br in ("cls", "reg"):
-        check("qn_" + br, bufs["qn_" + br][qrows], ref["qn_" + br][qrows])
-        for n in ("kn_", "vn_"):
-            check(n + br, bufs[n + br][:N], ref[n + br][:N])
-        vt, vt_ref = bufs["vt_" + br].view(B, 256, nk_pitch), ref["vt_" + br].view(B, 256, nk_pitch)
-        for b in range(B):
-            n, pad = clip_rows[b], min(((clip_rows[b] + 127) // 128) * 128, nk_pitch)
-            if n:
-                check(f"vt_{br}[clip {b}]", vt[b, :, :n], vt_ref[b, :, :n])
-            assert bool((vt[b, :, n:pad].view(torch.int16) == 0).all()), f"{case}: V^T pad of clip {b} is not zero"
-    check("x_ori cls", xo_c[:loc_total], rx_c[:loc_total])
-    check("x_ori reg", xo_r[:loc_total], rx_r[:loc_total])
+    def check(name, got, want, err_bound, scale, fused):
+        got = got.double()
+        assert not torch.isnan(got).any(), f"{case}: {name} has elements the projection never wrote"
+        bound = err_bound + u * want.abs() + 8 * 2.0 ** -24 * scale + (0.0 if fused else 2 * u * scale)
+        r = (got - want).abs() / bound
+        k = int(torch.argmax(r))
+        key = name.split(" (clip")[0]
+        worst[key] = max(worst.get(key, 0.0), float(r.reshape(-1)[k]))
+        assert float(r.reshape(-1)[k]) <= 1.0, (f"{case} / {dt}: {name} row {k // r.shape[1]} column {k % r.shape[1]}: "
+                                             f"{float(got.reshape(-1)[k]):.6g} vs {float(want.reshape(-1)[k]):.6g}, error "
+                                             f"{float(r.reshape(-1)[k]):.3g} x the bound")
+
+    for br, bank, w, ks in (("cls", bank_c, w_c, score), ("reg", bank_r, w_r, None)):
+        R = _reference(bank[:N], w, None if ks is None else ks[:N], 25.0)
+        qsel = qrows
+        for fused, got in ((True, bufs), (False, ref)):
+            tag = ("fused " if fused else "unfused ") + br
+            check(tag + " qn", got["qn_" + br][qsel], R["qn"][qsel], R["qn_err"][qsel], R["qn_scale"][qsel], fused)
+            for n in ("kn", "vn"):
+                check(f"{tag} {n}", got[f"{n}_{br}"][:N], R[n], R[n + "_err"], R[n + "_scale"], fused)
+            vt = got["vt_" + br].view(B, 256, nk_pitch)
+            for b in range(B):
+                n, pad = clip_rows[b], min(((clip_rows[b] + 127) // 128) * 128, nk_pitch)
+                if n:
+                    s0 = int(starts[b])
+                    check(f"{tag} V^T (clip {b})", vt[b, :, :n].T, R["v"][s0:s0 + n], R["v_err"][s0:s0 + n], 0.0, True)
+                assert bool((vt[b, :, n:pad].view(torch.int16) == 0).all()), f"{case}: {tag} V^T pad of clip {b} is not zero"
+        for fused, xo in ((True, xo_c if br == "cls" else xo_r), (False, rx_c if br == "cls" else rx_r)):
+            check(("fused " if fused else "unfused ") + br + " x_ori", xo[:loc_total], R["v"][qrows], R["v_err"][qrows], 0.0, True)
+    print(f"\n{case} / {dt}: worst error / bound " + ", ".join(f"{k} {v:.3f}" for k, v in worst.items()))
 
     # launches are deterministic: the same bytes in every element read downstream, also when the reg V^T / x_ori are off
     for other, xc_o, reg_vt in ((bufs2, xo_c2, True), (bufs3, xo_c3, False)):
