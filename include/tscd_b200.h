@@ -734,6 +734,88 @@ typedef struct {
 } tscd_repp_link_args;
 int tscd_repp_link(const tscd_repp_link_args* args, void* stream);
 
+/* ---- REPP bookkeeping after the linking (SURVEY.md section 8f-3) -----------------------------------------------------------
+ * The rest of REPP.__call__ on the device, exact to the bit (fp64 sums in the reference's order, no FMA contraction):
+ *   tscd_repp_prep       Predictor.to_repp_heavy (tools/val_to_imdb.py:193-218) on the packed table of tscd_pack_detections
+ *                        (packed with the resize ratios as scales) + the low-score filter / one-hot scores of REPP.__call__
+ *                        (REPP.py:247-256): compacted REPP detections in the layout tscd_repp_link reads.  Three kernels.
+ *   tscd_repp_tubelets   get_tubelets (REPP.py:138-190) and the unmatched lists (:109, :235-243) from the pairs of
+ *                        tscd_repp_link: a tubelet starts at every pair whose source has no incoming link, tubelets are numbered
+ *                        in [frame pair, extraction index] order; singletons follow (frames 0 .. n-2, detections without an
+ *                        outgoing link in ascending order, tubelet tails included).  Two kernels.
+ *   tscd_repp_emit       rescore_tubelets (:193-202), recoordinate_tubelets_full (:205-218) and tubelets_to_predictions
+ *                        (:221-233): the predictions table.  Three kernels.
+ * Detection rows ("data rows") hold one REPP detection each: box64 / kind / score / cls.  Position p of a video (the p-th frame key
+ * in the dict's insertion order, which is what get_tubelets and the unmatched singletons index) owns data rows
+ * [data_off[p], data_off[p] + data_cnt[p]); linking uses the frames in sorted order (frame_off).  For a video whose keys are
+ * already sorted both are the same (data_off / data_cnt NULL).
+ * Box kinds (the dtype np.array gives the members' boxes, which the convolution keeps): bit 1 = every coordinate a float32,
+ * bit 2 = every coordinate an integer, bit 4 = anything else; a tubelet's OR of 1 is float32, of 2 int64, otherwise float64.
+ * Device status codes (atomicMin): TSCD_ERR_CAPACITY when an output cap is too small, TSCD_ERR_INVALID_ARG when a class id is
+ * outside [0, num_classes) or a member / singleton index is outside its insertion-order frame (the reference's IndexError). */
+typedef struct {
+    int32_t num_frames, num_classes;
+    int32_t thr_f32;              /* 1: obj * cls >= min_tubelet_score compared in fp32 (NumPy 2 rules for a Python number), 0: fp64 */
+    double min_tubelet_score;
+    const float* packed;          /* [*, 12] tscd_pack_detections rows */
+    const int32_t* offsets;       /* [num_frames + 1] */
+    const int32_t* det_cand;      /* [num_frames]: 0 = frame without output (no detections) */
+    const int32_t* img_size;      /* [num_frames, 2] (height, width) */
+    int32_t* count;               /* workspace [num_frames] */
+    int32_t* frame_off;           /* out [num_frames + 1] */
+    float* bbox;                  /* out [N, 4] x, y, w, h (fp32, as tscd_repp_link reads them) */
+    float* center;                /* out [N, 2] normalised centre rounded to fp32 */
+    double* score;                /* out [N] obj * cls_score */
+    int32_t* cls;                 /* out [N] */
+    double* box64;                /* out [N, 4] the box as the dicts hold it (float32 or int coordinates), in fp64 */
+    int32_t* kind;                /* out [N] box kind bits */
+    int32_t* src;                 /* out [N] packed row of every detection */
+    int32_t* status;              /* [1] */
+} tscd_repp_prep_args;
+int tscd_repp_prep(const tscd_repp_prep_args* args, void* stream);
+
+typedef struct {
+    int32_t num_frames;
+    int32_t max_det;              /* pitch of `pairs` (as given to tscd_repp_link) */
+    int32_t add_unmatched;
+    int32_t cap;                  /* capacity of members / single / single_tub / tub_off - 1 (>= detections) */
+    const int32_t* frame_off;     /* [num_frames + 1] linking (sorted) order */
+    const int32_t* data_off;      /* [num_frames] or NULL (= frame_off) */
+    const int32_t* data_cnt;      /* [num_frames] or NULL (= frame_off differences) */
+    const int32_t* pairs;         /* [num_frames - 1, max_det, 2] */
+    const int32_t* pair_count;    /* [num_frames - 1] */
+    int32_t* next;                /* workspace [detections] */
+    int32_t* has_prev;            /* workspace [detections] */
+    int32_t* tail_of;             /* workspace [detections] */
+    int32_t* ws;                  /* workspace [2 * cap + num_frames + 1] */
+    int32_t* counts;              /* out [2]: tubelets, singletons */
+    int32_t* tub_off;             /* out [cap + 1]: tubelet t owns members[tub_off[t] .. tub_off[t+1]) */
+    int32_t* members;             /* out [cap] data rows in chain order */
+    int32_t* single;              /* out [cap] data rows of the singletons */
+    int32_t* single_tub;          /* out [cap] tubelet whose tail the singleton is, or -1 */
+    int32_t* status;              /* [1] */
+} tscd_repp_tubelets_args;
+int tscd_repp_tubelets(const tscd_repp_tubelets_args* args, void* stream);
+
+typedef struct {
+    int32_t num_frames, num_classes;
+    int32_t cap;                  /* as in tscd_repp_tubelets */
+    int32_t recoordinate;
+    double min_pred_score;
+    const double* window;         /* [2 * num_frames - 1] scipy.signal.windows.gaussian(2 * num_frames - 1, std), unnormalised */
+    const double* box64; const int32_t* kind; const double* score; const int32_t* cls;   /* data rows */
+    const int32_t* counts; const int32_t* tub_off; const int32_t* members; const int32_t* single; const int32_t* single_tub;
+    double* tub_score;            /* workspace [cap, num_classes] */
+    int32_t* tub_k;               /* workspace [cap] classes a tubelet emits */
+    double* mem_box;              /* workspace [cap, 4] re-coordinated member boxes */
+    int32_t* row_off;             /* workspace [2 * cap + 1] */
+    int64_t row_cap;              /* rows of `out` (2 * detections * num_classes always suffices) */
+    double* out;                  /* out [row_cap, 8]: data row, x, y, w, h, score, category, track id */
+    int32_t* n_out;               /* out [1] */
+    int32_t* status;              /* [1] */
+} tscd_repp_emit_args;
+int tscd_repp_emit(const tscd_repp_emit_args* args, void* stream);
+
 /* ---- long-clip mode: exchange of the global-frame bank rows between ranks (SURVEY.md section 8e) ----------------------
  * One clip sharded by frame: every rank runs K1-K3 on its own frames [n_local_frames local | n_global_frames global], then the
  * ranks all-gather ONE packed buffer each (ncclAllGather, issued by the host) and every rank builds the virtual clip

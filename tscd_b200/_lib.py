@@ -227,6 +227,23 @@ class ReppLinkArgs(C.Structure):
                 ("ws_pitch", C.c_int32), ("status", C.c_void_p)]
 
 
+class ReppPrepArgs(C.Structure):
+    _fields_ = [("num_frames", C.c_int32), ("num_classes", C.c_int32), ("thr_f32", C.c_int32), ("min_tubelet_score", C.c_double)] + \
+        _fields("packed:p offsets:p det_cand:p img_size:p count:p frame_off:p bbox:p center:p score:p cls:p box64:p kind:p src:p status:p")
+
+
+class ReppTubeletsArgs(C.Structure):
+    _fields_ = _fields("num_frames:i max_det:i add_unmatched:i cap:i frame_off:p data_off:p data_cnt:p pairs:p pair_count:p next:p "
+                       "has_prev:p tail_of:p ws:p counts:p tub_off:p members:p single:p single_tub:p status:p")
+
+
+class ReppEmitArgs(C.Structure):
+    _fields_ = [("num_frames", C.c_int32), ("num_classes", C.c_int32), ("cap", C.c_int32), ("recoordinate", C.c_int32),
+                ("min_pred_score", C.c_double)] + \
+        _fields("window:p box64:p kind:p score:p cls:p counts:p tub_off:p members:p single:p single_tub:p tub_score:p tub_k:p "
+                "mem_box:p row_off:p") + [("row_cap", C.c_int64)] + _fields("out:p n_out:p status:p")
+
+
 _lib = None
 
 # every symbol include/tscd_b200.h declares: (name, restype, argtypes)
@@ -264,6 +281,9 @@ SYMBOLS = [
     ("tscd_pack_detections", C.c_int, [C.POINTER(PackDetectionsArgs), C.c_void_p]),
     ("tscd_pack_rows", C.c_int, [C.POINTER(PackRowsArgs), C.c_void_p]),
     ("tscd_repp_link", C.c_int, [C.POINTER(ReppLinkArgs), C.c_void_p]),
+    ("tscd_repp_prep", C.c_int, [C.POINTER(ReppPrepArgs), C.c_void_p]),
+    ("tscd_repp_tubelets", C.c_int, [C.POINTER(ReppTubeletsArgs), C.c_void_p]),
+    ("tscd_repp_emit", C.c_int, [C.POINTER(ReppEmitArgs), C.c_void_p]),
     ("tscd_bank_pack_bytes", C.c_int64, [C.c_int32, C.c_int32]),
     ("tscd_bank_pack", C.c_int, [C.POINTER(BankPackArgs), C.c_void_p]),
     ("tscd_bank_unpack", C.c_int, [C.POINTER(BankUnpackArgs), C.c_void_p]),
@@ -291,7 +311,8 @@ def lib():
 
 # kernels launched per C-ABI call (for the bench's `gpu_launches` claim)
 _DEBUG_SYNC = os.environ.get("TSCD_DEBUG_SYNC", "0") == "1"
-KERNELS_PER_CALL = {"tscd_gather": 2, "tscd_nms_large": 3, "tscd_bank_unpack": 2, "tscd_clip_assemble": 2, "tscd_pack_detections": 2, "tscd_pack_rows": 2, "tscd_cafm_wide_p1": 2}
+KERNELS_PER_CALL = {"tscd_gather": 2, "tscd_nms_large": 3, "tscd_bank_unpack": 2, "tscd_clip_assemble": 2, "tscd_pack_detections": 2, "tscd_pack_rows": 2, "tscd_cafm_wide_p1": 2,
+                    "tscd_repp_prep": 3, "tscd_repp_tubelets": 2, "tscd_repp_emit": 3}
 launch_count = 0
 # optional per-entry-point CUDA-event timing: {"names": set or None (= all), "events": {name: [(start, end), ...]}}
 profile = None
