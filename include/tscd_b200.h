@@ -906,6 +906,38 @@ typedef struct {
 } tscd_clip_assemble_args;
 int tscd_clip_assemble(const tscd_clip_assemble_args* args, void* stream);
 
+/* ---- video pack: the detections of whole videos from several clip calls, in frame order (tscd_b200/video.py) ----------------
+ * A group of videos runs as several clip calls (tscd_clip_assemble + the stage); each call leaves padded detection rows
+ * [n_rows, cap, 7] + counts for its B * L local frames.  tscd_video_pack writes, in ONE pass, the tscd_pack_detections table of
+ * every video of the group back to back: frame i of the group (video-major, frame-minor) takes the rows of call map[i].call,
+ * local row map[i].row; the packed row's frame column is map[i].frame (the frame's index in its video), so the rows of one video
+ * equal tscd_pack_detections over that video's frames in order (same per-row arithmetic: the shared device function).  Frames
+ * the clips repeat (the padded tail of a video's last clip) are simply not in the map.  Two kernels: a one-CTA scan of the counts
+ * into offsets, then one CTA per frame.  A map entry outside the calls contributes no rows and sets status to
+ * TSCD_ERR_INVALID_ARG.  det_cand (optional) receives the frames' candidate counts (0 = the reference's None). */
+typedef struct {
+    const float* rows;           /* [n_rows, cap, 7] det_rows (or ori_rows) of one clip call */
+    const int32_t* count;        /* [n_rows] */
+    const int32_t* cand;         /* [n_rows] candidate counts (det_cand) or NULL */
+    int32_t n_rows;              /* B * L of the call */
+    int32_t pad;
+} tscd_video_pack_call;
+
+typedef struct {
+    int32_t num_frames;          /* frames of the group (all videos) */
+    int32_t num_calls;
+    int32_t cap;                 /* row pitch of every call's rows */
+    int32_t pad;
+    const tscd_video_pack_call* calls;   /* DEVICE array [num_calls] */
+    const int32_t* map;          /* [num_frames, 3]: call, row of that call, frame index inside its video */
+    const float* scale;          /* [num_frames] resize scale (boxes are DIVIDED by it), or NULL */
+    int32_t* offsets;            /* out [num_frames + 1] */
+    float* packed;               /* out [num_frames * cap, 12] */
+    int32_t* det_cand;           /* out [num_frames] or NULL */
+    int32_t* status;             /* [1] or NULL */
+} tscd_video_pack_args;
+int tscd_video_pack(const tscd_video_pack_args* args, void* stream);
+
 /* Debug aid: cycles block 0 of the last tscd_cafm_chain launches spent per phase
  * (0 assignment re-index, 1 query input, 2 q projection, 3 normalise, 4 attention, 5 norms/state, 6 state carry). */
 int tscd_debug_chain_clocks(long long* host_out8, int reset);

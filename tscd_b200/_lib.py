@@ -13,6 +13,7 @@ MAX_LEVELS = 3
 _ERR = {-1: "invalid argument", -2: "unsupported configuration", -3: "capacity exceeded", -4: "CUDA error",
         -5: "frame-store slot out of range or never written"}
 TSCD_ERR_CAPACITY, TSCD_ERR_FRAME_SLOT = -3, -5
+TSCD_ERR_INVALID_ARG = -1
 
 
 class View(C.Structure):
@@ -219,6 +220,14 @@ class PackRowsArgs(C.Structure):
     _fields_ = _fields("num_frames:i cap:i rows:p count:p offsets:p packed:p")
 
 
+class VideoPackCall(C.Structure):
+    _fields_ = _fields("rows:p count:p cand:p n_rows:i pad:i")
+
+
+class VideoPackArgs(C.Structure):
+    _fields_ = _fields("num_frames:i num_calls:i cap:i pad:i calls:p map:p scale:p offsets:p packed:p det_cand:p status:p")
+
+
 class ReppLinkArgs(C.Structure):
     _fields_ = [("num_frames", C.c_int32), ("max_det", C.c_int32), ("distance_func", C.c_int32), ("clf_mode", C.c_int32),
                 ("clf_thr", C.c_double), ("coef", C.c_double * 4), ("intercept", C.c_double),
@@ -289,6 +298,7 @@ SYMBOLS = [
     ("tscd_bank_unpack", C.c_int, [C.POINTER(BankUnpackArgs), C.c_void_p]),
     ("tscd_frame_scatter", C.c_int, [C.POINTER(FrameScatterArgs), C.c_void_p]),
     ("tscd_clip_assemble", C.c_int, [C.POINTER(ClipAssembleArgs), C.c_void_p]),
+    ("tscd_video_pack", C.c_int, [C.POINTER(VideoPackArgs), C.c_void_p]),
 ]
 
 
@@ -311,7 +321,7 @@ def lib():
 
 # kernels launched per C-ABI call (for the bench's `gpu_launches` claim)
 _DEBUG_SYNC = os.environ.get("TSCD_DEBUG_SYNC", "0") == "1"
-KERNELS_PER_CALL = {"tscd_gather": 2, "tscd_nms_large": 3, "tscd_bank_unpack": 2, "tscd_clip_assemble": 2, "tscd_pack_detections": 2, "tscd_pack_rows": 2, "tscd_cafm_wide_p1": 2,
+KERNELS_PER_CALL = {"tscd_gather": 2, "tscd_nms_large": 3, "tscd_bank_unpack": 2, "tscd_clip_assemble": 2, "tscd_pack_detections": 2, "tscd_pack_rows": 2, "tscd_video_pack": 2, "tscd_cafm_wide_p1": 2,
                     "tscd_repp_prep": 3, "tscd_repp_tubelets": 2, "tscd_repp_emit": 3}
 launch_count = 0
 # optional per-entry-point CUDA-event timing: {"names": set or None (= all), "events": {name: [(start, end), ...]}}

@@ -95,6 +95,16 @@ __device__ __forceinline__ int block_excl_scan(int v, int* scratch, int* total) 
     return res;
 }
 
+// One packed detection row (tscd_pack_detections, tscd_video_pack): stage row r = [x1,y1,x2,y2,obj,cls_score,cls] of frame
+// `frame`, resize scale s -> d = [frame, x1/s, y1/s, (x2/s - x1/s), (y2/s - y1/s), obj * cls, class, obj, x2/s, y2/s, cls_score, 0]
+// (the reference's operation order: divide, then subtract; explicit rounding, no contraction).
+__device__ __forceinline__ void pack_detection_row(const float* r, float frame, float s, float* d) {
+    const float x1 = __fdiv_rn(r[0], s), y1 = __fdiv_rn(r[1], s), x2 = __fdiv_rn(r[2], s), y2 = __fdiv_rn(r[3], s);
+    d[0] = frame; d[1] = x1; d[2] = y1; d[3] = __fsub_rn(x2, x1); d[4] = __fsub_rn(y2, y1);
+    d[5] = __fmul_rn(r[4], r[5]); d[6] = r[6]; d[7] = r[4];
+    d[8] = x2; d[9] = y2; d[10] = r[5]; d[11] = 0.f;
+}
+
 // ---- block-wide bitonic sort, descending, 64-bit keys ---------------------------------------------------
 // E keys per thread in registers (element index = tid * E + r, E * blockDim.x keys in total, both powers of two).
 // Compare-exchange distances below E stay inside the thread, distances below 32 * E go through warp shuffles, only

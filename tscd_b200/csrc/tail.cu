@@ -438,14 +438,8 @@ __global__ void pack_detections_kernel(const tscd_pack_detections_args a) {
     const int n = min(a.count[f], a.cap);
     const int o = a.offsets[f];
     const float s = a.scale ? a.scale[f] : 1.f;
-    for (int j = threadIdx.x; j < n; j += blockDim.x) {
-        const float* r = a.rows + ((int64_t)f * a.cap + j) * 7;
-        float* d = a.packed + (int64_t)(o + j) * 12;
-        const float x1 = __fdiv_rn(r[0], s), y1 = __fdiv_rn(r[1], s), x2 = __fdiv_rn(r[2], s), y2 = __fdiv_rn(r[3], s);
-        d[0] = (float)f; d[1] = x1; d[2] = y1; d[3] = __fsub_rn(x2, x1); d[4] = __fsub_rn(y2, y1);
-        d[5] = __fmul_rn(r[4], r[5]); d[6] = r[6]; d[7] = r[4];
-        d[8] = x2; d[9] = y2; d[10] = r[5]; d[11] = 0.f;
-    }
+    for (int j = threadIdx.x; j < n; j += blockDim.x)
+        pack_detection_row(a.rows + ((int64_t)f * a.cap + j) * 7, (float)f, s, a.packed + (int64_t)(o + j) * 12);
 }
 
 // raw variant: the [n,7] rows themselves, frame after frame (forward_host's single read-back)

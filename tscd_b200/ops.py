@@ -571,3 +571,37 @@ def clip_assemble(store, clip_slots: torch.Tensor, B: int, F: int, Lf: int, row_
          bank_reg=out["bank_reg"], bank_edge=out["bank_edge"], bank_score=out["bank_score"], sel_idx=out.get("sel_idx"),
          sel_rows=out["sel_rows"], status=status)
     return out
+
+
+# ----------------------------------------------------------------------------------------------- video pack
+def video_pack(calls, frame_map: torch.Tensor, scale: Optional[torch.Tensor] = None, status: Optional[torch.Tensor] = None,
+               out: Optional[dict] = None) -> dict:
+    """tscd_video_pack: calls = [(rows [n, cap, 7], count [n], cand [n] or None), ...] (device tensors of the clip calls of a
+    group), frame_map [frames, 3] int32 device tensor of (call, row, frame index in its video), scale [frames] fp32 or None.
+    Returns {'packed' [frames * cap, 12], 'offsets' [frames + 1], 'det_cand' [frames], 'calls' (the device call array, kept
+    alive with the launch)}; no host sync.  `out`: preallocated buffers of those shapes."""
+    if not calls:
+        raise RuntimeError("video_pack: no clip calls")
+    cap = calls[0][0].shape[1]
+    for rows, count, cand in calls:
+        if rows.dim() != 3 or rows.shape[1] != cap or rows.shape[2] != 7 or rows.dtype != torch.float32 or not rows.is_contiguous():
+            raise RuntimeError(f"video_pack: every call's rows must be contiguous fp32 [n, {cap}, 7], got {tuple(rows.shape)}")
+        if count.dtype != torch.int32 or count.numel() < rows.shape[0]:
+            raise RuntimeError("video_pack: counts must be int32 with one entry per row")
+    dev = frame_map.device
+    nf = frame_map.shape[0]
+    arr = (L.VideoPackCall * len(calls))()
+    for i, (rows, count, cand) in enumerate(calls):
+        arr[i].rows, arr[i].count, arr[i].cand, arr[i].n_rows = _p(rows), _p(count), _p(cand), rows.shape[0]
+    # the call array travels to the device with the launch (a pinned copy: stream-ordered, the host buffer is kept by torch
+    # until the copy has run)
+    host = torch.frombuffer(bytearray(C.string_at(arr, C.sizeof(arr))), dtype=torch.uint8).pin_memory()
+    dcalls = host.to(dev, non_blocking=True)
+    if out is None:
+        out = dict(packed=torch.empty(max(nf * cap, 1), 12, dtype=torch.float32, device=dev),
+                   offsets=torch.empty(nf + 1, dtype=torch.int32, device=dev),
+                   det_cand=torch.empty(nf, dtype=torch.int32, device=dev))
+    call("tscd_video_pack", L.VideoPackArgs, num_frames=nf, num_calls=len(calls), cap=cap, pad=0, calls=dcalls, map=frame_map,
+         scale=scale, offsets=out["offsets"], packed=out["packed"], det_cand=out["det_cand"], status=status)
+    out["calls"] = dcalls
+    return out
